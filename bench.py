@@ -6,6 +6,7 @@ dominant kernel, the same path end-to-end through host buffers, and the referenc
 
     python bench.py --gpus N --steps K --warmup W            # our arm (torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  # reference CPU arm (rank 0 only)
+    python bench.py --steps K --dump-outputs DIR             # also write the last timed step's features
 
 Prints ONE JSON line on rank 0.
 """
@@ -25,6 +26,20 @@ if ROOT not in sys.path:
 UTT_LEN = 64600
 TRAFFIC_FILE = os.path.join(ROOT, "profiles", "r2_traffic.json")   # written by tools/ncu_summary.py from ncu --set full captures
 SEED = 1234  # the reference's default seed (maze5.py:449)
+DUMP_BYTES = 60_000_000  # --dump-outputs stays under 64 MB, .npy header included
+
+
+def dump_outputs(out, directory):
+    """Rank 0's features of the last timed step as DIR/features.npy (float32).  A batch larger than DUMP_BYTES is
+    written as a seeded sample of whole utterances, kept in batch order, so two builds can be compared row for row."""
+    import numpy as np
+    import torch
+    n = min(out.shape[0], DUMP_BYTES // (out[0].numel() * out.element_size()))
+    rows = np.sort(np.random.RandomState(SEED).choice(out.shape[0], n, replace=False))
+    sample = out.index_select(0, torch.from_numpy(rows).to(out.device)).cpu().numpy()
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "features.npy"), sample)
+
 
 WORKLOADS = {
     # BASELINE.json configs[1]: the configuration the metric is quoted on
@@ -300,7 +315,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-config4", action="store_true")
     ap.add_argument("--cpu-budget", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the features of the last timed step to DIR/features.npy (float32, under 64 MB: a seeded "
+                         "sample of utterances when the batch is larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the b200 arm")
     # torchrun exports OMP_NUM_THREADS=1 to every rank; rank 0 also times the reference CPU path on ALL host cores
     # (cpu_baseline / the reference arm), so its OpenMP / MKL runtimes must start with all of them (before torch loads)
     if int(os.environ.get("RANK", "0")) == 0:
@@ -397,6 +419,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     elapsed_ms = float(t.item())
     ms_per_step = elapsed_ms / K
+    if args.dump_outputs and rank == 0:
+        dump_outputs(outs[(K - 1) % n_sets], args.dump_outputs)
     value = world * B * K / (elapsed_ms / 1000.0)
 
     # ---- end to end through host buffers (pinned), copies inside the timed region ----
