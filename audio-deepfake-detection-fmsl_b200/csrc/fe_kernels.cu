@@ -8,6 +8,9 @@
 #include <math.h>
 #include <stdlib.h>
 #include <atomic>
+#include <map>
+#include <mutex>
+#include <utility>
 
 #include "fe_fft.cuh"
 #include "fe_tail.cuh"
@@ -1013,27 +1016,27 @@ __global__ void __launch_bounds__(256) fe_tail_pointwise_kernel(fe_tail_args a) 
 
 cudaError_t set_smem(const void* fn, size_t bytes) {
   if (bytes <= 32 * 1024) return cudaSuccess;   // the 48 KB default covers static + dynamic: opt in well below it
-  // The opt-in belongs to (function, device); it costs a microsecond or two per call, which a small-batch launch
-  // notices.  Each host thread remembers the largest size it has been granted per (function, device).
-  struct granted { const void* fn; int dev; size_t bytes; };
-  constexpr int kSlots = 16;
-  thread_local granted cache[kSlots] = {};
-  thread_local int next = 0;
-  const int dev = fe_current_device();
-  for (int i = 0; i < kSlots; ++i)
-    if (cache[i].fn == fn && cache[i].dev == dev && cache[i].bytes >= bytes) return cudaSuccess;
-  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e == cudaSuccess && dev >= 0) {
-    int at = -1;
-    for (int i = 0; i < kSlots; ++i)
-      if (cache[i].fn == fn && cache[i].dev == dev) at = i;
-    if (at < 0) { at = next; next = (next + 1) % kSlots; }
-    cache[at] = granted{fn, dev, bytes};
-  }
-  return e;
+  return fe_ensure_smem(fn, bytes);
 }
 
 }  // namespace
+
+cudaError_t fe_ensure_smem(const void* fn, size_t bytes) {
+  // The opt-in is process-wide per (function, device), and it costs a microsecond or two per call, which a small-batch
+  // launch notices.  The largest size granted so far is kept per (function, device) under one lock: two host threads
+  // launching the same kernel with different sizes must not lower the attribute below what the other was granted
+  // (its launch would then be rejected), so a smaller request never calls cudaFuncSetAttribute.
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> granted;
+  const int dev = fe_current_device();
+  if (dev < 0) return cudaErrorInvalidDevice;
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& have = granted[{fn, dev}];
+  if (have >= bytes) return cudaSuccess;
+  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e == cudaSuccess) have = bytes;
+  return e;
+}
 
 int fe_current_device(void) {
   int dev = -1;

@@ -46,6 +46,10 @@ struct fe_tail_args {
 constexpr int kFeMaxDevices = 64;
 int fe_current_device(void);        // cudaGetDevice, -1 on error
 int fe_device_sms(int dev);         // multiprocessor count of `dev`
+// Opts kernel `fn` in to `bytes` of dynamic shared memory on the current device.  Process-wide and thread-safe: the
+// attribute is never set below the largest size granted so far for (fn, device); an already granted size costs one
+// uncontended lock and no CUDA call.
+cudaError_t fe_ensure_smem(const void* fn, size_t bytes);
 
 // A ragged clip the streaming kernel can read where it lies: pad() only truncates it (len >= T), and its first sample
 // is 16-byte aligned relative to the tensor map's base and within the map's reach (32 steps of 32 GB above the base).

@@ -824,13 +824,8 @@ cudaError_t fe_stream_launch(const b200fe_params* p, const fe_fft_args& fa, int6
   const int dev = fe_current_device();
   if (dev < 0) return cudaErrorInvalidDevice;
   {
-    // the opt-in is per device (context): remembered per device ordinal, largest size granted so far
-    static std::atomic<int> attr_done[kFeMaxDevices];
-    if (dev >= kFeMaxDevices || attr_done[dev].load(std::memory_order_relaxed) < smem) {
-      cudaError_t e = cudaFuncSetAttribute(fe_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-      if (e != cudaSuccess) return e;
-      if (dev < kFeMaxDevices) attr_done[dev].store(smem, std::memory_order_relaxed);
-    }
+    cudaError_t e = fe_ensure_smem((const void*)fe_stream_kernel, (size_t)smem);
+    if (e != cudaSuccess) return e;
   }
   const int sms = fe_device_sms(dev);
   const int grid = a.n_tiles < sms ? a.n_tiles : sms;

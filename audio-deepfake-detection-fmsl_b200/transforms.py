@@ -19,6 +19,8 @@ from __future__ import annotations
 
 import ctypes as C
 import math
+import threading
+from collections import OrderedDict
 from typing import Callable, Dict, Optional, Tuple
 
 import numpy as np
@@ -122,8 +124,10 @@ def _as_f32_ptr(t: Optional[Tensor]):
 # --------------------------------------------------------------------------------------------
 class FrontEndEngine:
     """Owns a ``b200fe_params``, the packed constant-table blob and the device-side caches
-    (uploaded blob, grow-only workspace) of one transform configuration.  All buffers are torch
-    tensors: the C library allocates nothing."""
+    (uploaded blob, one grow-only workspace per stream) of one transform configuration.  All buffers are torch
+    tensors: the C library allocates nothing.  Several host threads and streams may share one engine."""
+
+    WORKSPACES_PER_DEVICE = 8
 
     def __init__(self, *, n_fft: int, win_length: int, hop_length: int, window: Tensor,
                  fbank: Optional[Tensor], dct: Optional[Tensor], log_mode: int, top_db: Optional[float],
@@ -159,7 +163,15 @@ class FrontEndEngine:
         self.requested_variant = variant
         p.variant = resolved
         self._blob_dev: Dict[torch.device, Tensor] = {}
-        self._workspace: Dict[torch.device, Tensor] = {}
+        # device -> {stream handle -> workspace}, least recently used first (see workspace_on)
+        self._workspace: Dict[torch.device, "OrderedDict[int, Tensor]"] = {}
+        self._host_staging: Dict[torch.device, Tuple[Tensor, list]] = {}
+        # _lock: held from choosing the workspace to the return of the enqueueing C call, so that two host threads on
+        # one stream cannot interleave their launch sequences; _host_lock: serialises features_host calls (which block
+        # until their copies are done, and must not hold up device-path callers); _tables_lock: first upload only
+        self._lock = threading.Lock()
+        self._host_lock = threading.Lock()
+        self._tables_lock = threading.Lock()
 
     # -- queries ---------------------------------------------------------------------------------
     def n_frames(self, T: int) -> int:
@@ -187,15 +199,35 @@ class FrontEndEngine:
     def tables_on(self, device: torch.device) -> Tensor:
         t = self._blob_dev.get(device)
         if t is None:
-            t = torch.from_numpy(self._blob_host).to(device)
-            self._blob_dev[device] = t
+            with self._tables_lock:
+                t = self._blob_dev.get(device)
+                if t is None:
+                    t = torch.from_numpy(self._blob_host).to(device)   # (a synchronous copy: usable from any stream)
+                    self._blob_dev[device] = t
         return t
 
-    def workspace_on(self, device: torch.device, nbytes: int) -> Tensor:
-        t = self._workspace.get(device)
-        if t is None or t.numel() < nbytes:
-            t = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=device)
-            self._workspace[device] = t
+    def workspace_on(self, device: torch.device, nbytes: int, stream: int) -> Tensor:
+        """Workspace of at least ``nbytes`` for a call enqueued on ``stream``, the current stream of ``device`` (the
+        caller holds ``_lock`` and has made ``device`` current).  One workspace per stream: calls on different streams
+        may overlap on the GPU, and each keeps group maxima and filterbank energies in it between kernels.  A workspace
+        is allocated while its stream is current, so the caching allocator reuses its block, once it is dropped (grown,
+        or evicted from the per-device cache of WORKSPACES_PER_DEVICE streams), only in that stream's order.  During
+        stream capture a fresh, uncached workspace is allocated: it belongs to the graph's private memory pool for the
+        graph's lifetime, and no later eager call or other graph writes into it."""
+        if torch.cuda.is_current_stream_capturing():
+            return torch.empty(max(nbytes, 256), dtype=torch.uint8, device=device)
+        per_dev = self._workspace.get(device)
+        t = None if per_dev is None else per_dev.get(stream)
+        if t is not None and t.numel() >= nbytes:
+            per_dev.move_to_end(stream)
+            return t
+        if per_dev is None:
+            per_dev = self._workspace[device] = OrderedDict()
+        per_dev.pop(stream, None)
+        t = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=device)
+        per_dev[stream] = t
+        while len(per_dev) > self.WORKSPACES_PER_DEVICE:
+            per_dev.popitem(last=False)
         return t
 
     def _params_with_group(self, group: int) -> _lib.Params:
@@ -264,7 +296,7 @@ class FrontEndEngine:
                 raise ValueError("offsets / lengths must be on the waveform's device")
             if lengths.numel() != R or R < 1:
                 raise ValueError("offsets and lengths must have the same, non-zero number of entries")
-            if validate:
+            if validate and not torch.cuda.is_current_stream_capturing():   # (.tolist() cannot run in a capture)
                 l64 = lengths.to(torch.int64)
                 bad = torch.stack([(l64 < 1).any(), (offsets < 0).any(), ((offsets + l64) > wave2d.numel()).any()])
                 bad = bad.tolist()
@@ -281,16 +313,17 @@ class FrontEndEngine:
         ws_bytes = wc.get(wkey)
         if ws_bytes is None:
             ws_bytes = wc[wkey] = _lib.check(self.lib.b200fe_workspace_bytes_ex(C.byref(p), R, T, 0 if offsets is None else 1))
-        ws = self.workspace_on(dev, ws_bytes)
 
         def launch():
             stream = torch.cuda.current_stream(dev).cuda_stream
-            _lib.check(self.lib.b200fe_features_forward(
-                wave2d.data_ptr(), R, T,
-                None if offsets is None else offsets.data_ptr(),
-                None if lengths is None else lengths.data_ptr(),
-                C.byref(p), self.tables_on(dev).data_ptr(), out.data_ptr(), ws.data_ptr(), ws.numel(),
-                C.c_void_p(stream)))
+            with self._lock:
+                ws = self.workspace_on(dev, ws_bytes, stream)
+                _lib.check(self.lib.b200fe_features_forward(
+                    wave2d.data_ptr(), R, T,
+                    None if offsets is None else offsets.data_ptr(),
+                    None if lengths is None else lengths.data_ptr(),
+                    C.byref(p), self.tables_on(dev).data_ptr(), out.data_ptr(), ws.data_ptr(), ws.numel(),
+                    C.c_void_p(stream)))
         if torch.cuda.current_device() == (dev.index if dev.index is not None else torch.cuda.current_device()):
             launch()                       # (the device guard costs a few microseconds per call)
         else:
@@ -309,9 +342,9 @@ class FrontEndEngine:
             out = torch.empty((R, self.params.n_filter, nf), dtype=torch.float32, device=dev)
         p = self._params_for_call(self.params, T, wave2d.data_ptr(), False)
         ws_bytes = _lib.check(self.lib.b200fe_workspace_bytes(C.byref(p), R, T))
-        ws = self.workspace_on(dev, ws_bytes)
-        with torch.cuda.device(dev):
+        with torch.cuda.device(dev), self._lock:
             stream = torch.cuda.current_stream(dev).cuda_stream
+            ws = self.workspace_on(dev, ws_bytes, stream)
             _lib.check(self.lib.b200fe_fbank_energies_forward(
                 wave2d.data_ptr(), R, T, None, None, C.byref(p), self.tables_on(dev).data_ptr(),
                 out.data_ptr(), ws.data_ptr(), ws.numel(), C.c_void_p(stream)))
@@ -321,7 +354,8 @@ class FrontEndEngine:
                       chunk_rows: int = 512, n_streams: int = 3) -> Tensor:
         """End-to-end path: HOST ``(R,T)`` float32 — or int16 PCM, converted ``x / 32768`` on the device so that only
         half the bytes cross PCIe — (ideally pinned) in, HOST features out, with the host<->device copies
-        pipelined against the kernels inside the library (``b200fe_features_forward_host[_i16]``)."""
+        pipelined against the kernels inside the library (``b200fe_features_forward_host[_i16]``).  The staging
+        buffer and the copy streams belong to the engine: calls on one engine from several threads run one at a time."""
         if wave_host.device.type != "cpu" or wave_host.dtype not in (torch.float32, torch.int16) or wave_host.dim() != 2:
             raise TypeError("features_host expects a 2-D float32 (or int16 PCM) CPU tensor")
         pcm16 = wave_host.dtype == torch.int16
@@ -336,24 +370,21 @@ class FrontEndEngine:
         p = self._params_for_call(self.params, T, None, False)   # staged rows are 256-byte aligned
         sizer = self.lib.b200fe_host_staging_bytes_i16 if pcm16 else self.lib.b200fe_host_staging_bytes
         need = _lib.check(sizer(C.byref(p), chunk_rows, T, n_streams))
-        key = ("host", device)
-        st = self._workspace.get(key)
-        if st is None or st.numel() < need:
-            st = torch.empty(need, dtype=torch.uint8, device=device)
-            self._workspace[key] = st
-        skey = ("streams", device)
-        streams = self._workspace.get(skey)
-        if streams is None or len(streams) < n_streams:
-            streams = [torch.cuda.Stream(device=device) for _ in range(4)]
-            self._workspace[skey] = streams
-        arr = (C.c_void_p * n_streams)(*[s.cuda_stream for s in streams[:n_streams]])
-        with torch.cuda.device(device):
-            tables = self.tables_on(device)
-            torch.cuda.current_stream(device).synchronize()  # tables upload finished
-            call = self.lib.b200fe_features_forward_host_i16 if pcm16 else self.lib.b200fe_features_forward_host
-            _lib.check(call(
-                wave_host.data_ptr(), R, T, C.byref(p), tables.data_ptr(), out_host.data_ptr(),
-                st.data_ptr(), st.numel(), chunk_rows, arr, n_streams))
+        with self._host_lock:
+            st, streams = self._host_staging.get(device, (None, None))
+            if st is None or st.numel() < need:
+                if streams is None:
+                    streams = [torch.cuda.Stream(device=device) for _ in range(4)]
+                st = torch.empty(need, dtype=torch.uint8, device=device)
+                self._host_staging[device] = (st, streams)
+            arr = (C.c_void_p * n_streams)(*[s.cuda_stream for s in streams[:n_streams]])
+            with torch.cuda.device(device):
+                tables = self.tables_on(device)
+                torch.cuda.current_stream(device).synchronize()  # tables upload finished
+                call = self.lib.b200fe_features_forward_host_i16 if pcm16 else self.lib.b200fe_features_forward_host
+                _lib.check(call(
+                    wave_host.data_ptr(), R, T, C.byref(p), tables.data_ptr(), out_host.data_ptr(),
+                    st.data_ptr(), st.numel(), chunk_rows, arr, n_streams))
         return out_host
 
 

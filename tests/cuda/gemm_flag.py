@@ -12,7 +12,7 @@ R = int(sys.argv[1]) if len(sys.argv) > 1 else 2
 x = (0.1 * torch.randn(R, 64600, device="cuda")).clamp_(-1, 1)
 e = eng.fbank_energies(x)
 torch.cuda.synchronize()
-ws = eng._workspace[x.device]
+ws = eng._workspace[x.device][torch.cuda.current_stream().cuda_stream]   # the current stream's workspace
 nbytes = eng.lib.b200fe_workspace_bytes(C.byref(eng.params), R, 64600)
 flag = ws[nbytes - 65536: nbytes - 65536 + 4].cpu().numpy().view(np.int32)[0]
 print("timeout flag:", flag, "(0 = none; else code*1000 + warp)")

@@ -13,7 +13,7 @@ x = (0.1 * torch.randn(R, 64600, device="cuda")).clamp_(-1, 1)
 for _ in range(2):
     e = eng.fbank_energies(x)
 torch.cuda.synchronize()
-ws = eng._workspace[x.device]
+ws = eng._workspace[x.device][torch.cuda.current_stream().cuda_stream]   # the current stream's workspace
 nbytes = eng.lib.b200fe_workspace_bytes(C.byref(eng.params), R, 64600)
 tail = ws[nbytes - 65536: nbytes].cpu().numpy()
 tr = np.frombuffer(tail[256:256 + 8 * 8 * 16 * 8].tobytes(), dtype=np.int64).reshape(8, 8, 16)

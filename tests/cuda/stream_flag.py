@@ -16,7 +16,7 @@ try:
     print("ok")
 except Exception as ex:
     print("error:", str(ex)[:100])
-ws = eng._workspace[x.device]
+ws = eng._workspace[x.device][torch.cuda.current_stream().cuda_stream]   # the current stream's workspace
 nbytes = eng.lib.b200fe_workspace_bytes(C.byref(eng.params), R, 64600)
 try:
     tail = ws[nbytes - 65536: nbytes - 65536 + 16].cpu().numpy()

@@ -20,7 +20,7 @@ for i in range(N):
 t1.record()
 torch.cuda.synchronize()
 print("last launch: %.3f ms" % t0.elapsed_time(t1))
-ws = eng._workspace[x.device]
+ws = eng._workspace[x.device][torch.cuda.current_stream().cuda_stream]   # the current stream's workspace
 nbytes = eng.lib.b200fe_workspace_bytes(C.byref(eng.params), R, 64600)
 tail = ws[nbytes - 65536: nbytes].cpu().numpy()
 print("flag", tail[:4].view(np.int32)[0])

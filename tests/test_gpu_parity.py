@@ -1,6 +1,7 @@
 """Parity of the CUDA path (called through the C-ABI via the drop-in modules) against the committed
 golden vectors, the reference CPU path (torchaudio, live) and the oracle restatement.  Needs a B200."""
 import ctypes as C
+from collections import OrderedDict
 
 import numpy as np
 import pytest
@@ -273,9 +274,10 @@ print("chunks-ok")
     assert r.returncode == 0 and "chunks-ok" in r.stdout, r.stdout + r.stderr
 
 
-def test_ragged_in_place_far_apart_buffers(fe):
-    """The ragged tensor maps reach 32 GB steps above their base: the flat clip buffer and the engine's workspace may
-    lie tens of GB apart.  Both are carved out of one 40 GB allocation here, 39 GB apart, in either order."""
+def test_ragged_in_place_far_from_the_stream_workspace(fe):
+    """The ragged tensor maps reach 32 GB steps above their base: the flat clip buffer and the workspace of the stream
+    the call runs on may lie tens of GB apart.  Both are carved out of one 40 GB allocation here, 39 GB apart, in
+    either order; the workspace is seeded as the current stream's entry of the engine's per-stream cache."""
     free, _ = torch.cuda.mem_get_info()
     if free < 50 << 30:
         pytest.skip("needs ~45 GB of free device memory")
@@ -293,9 +295,10 @@ def test_ragged_in_place_far_apart_buffers(fe):
         flat_d = flat_part[: flat.nbytes].view(torch.float32)
         flat_d.copy_(torch.from_numpy(flat))
         m.engine._workspace.clear()
-        m.engine._workspace[flat_d.device] = ws_part[: 1 << 30] if ws_part is hi else ws_part[32 << 20:]
+        key = torch.cuda.current_stream(dev()).cuda_stream        # the workspace of the stream the call runs on
+        m.engine._workspace[flat_d.device] = OrderedDict({key: ws_part[: 1 << 30] if ws_part is hi else ws_part[32 << 20:]})
         got = m.forward_ragged(flat_d, cuda(offsets), cuda(lens), 64600)
-        ws = m.engine._workspace[flat_d.device]
+        ws = m.engine._workspace[flat_d.device][key]
         assert abs(ws.data_ptr() - flat_d.data_ptr()) > 32 << 30     # the engine kept the seeded workspace
         assert torch.equal(got, want)
     m.engine._workspace.clear()
