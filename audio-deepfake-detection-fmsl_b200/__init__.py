@@ -14,6 +14,7 @@ from .transforms import (ComputeDeltas, FrontEndEngine, LFCC, LFCCDelta, MelSpec
                          create_dct, linear_fbanks, melscale_fbanks, pack_clips)
 from .maze import LFCC_FILTS, FeatureSlot, MazeScorer, fill_deterministic
 from .evaluation import eer_min_dcf, eer_min_dcf_device, gather_scores, shard_range, write_score_file
+from .sweep import score_host_pcm, score_host_ragged
 
 # names SURVEY.md 8(b) uses for the drop-in modules
 B200LFCC = LFCC
@@ -28,4 +29,5 @@ __all__ = [
     "linear_fbanks", "melscale_fbanks", "create_dct", "pack_clips",
     "MazeScorer", "FeatureSlot", "LFCC_FILTS", "fill_deterministic",
     "shard_range", "gather_scores", "eer_min_dcf", "eer_min_dcf_device", "write_score_file",
+    "score_host_pcm", "score_host_ragged",
 ]

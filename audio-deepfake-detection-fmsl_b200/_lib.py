@@ -83,6 +83,13 @@ _SIGNATURES = {
     "b200fe_host_staging_bytes_i16": (C.c_int64, [_P, C.c_int64, C.c_int64, C.c_int32]),
     "b200fe_features_forward_host_i16": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int64, _P, C.c_void_p, C.c_void_p,
                                                      C.c_void_p, C.c_size_t, C.c_int64, C.POINTER(C.c_void_p), C.c_int32]),
+    "b200fe_workspace_bytes_ragged_i16": (C.c_int64, [_P, C.c_int64, C.c_int64]),
+    "b200fe_features_forward_ragged_i16": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, _P,
+                                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "b200fe_host_staging_bytes_ragged": (C.c_int64, [_P, C.c_int64, C.c_int64, C.c_int32, C.c_int32]),
+    "b200fe_features_forward_host_ragged": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p,
+                                                        C.c_int64, C.c_int64, _P, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                        C.c_size_t, C.c_int64, C.POINTER(C.c_void_p), C.c_int32]),
     "b200fe_eer_workspace_bytes": (C.c_int64, [C.c_int64]),
     "b200fe_eer_min_dcf": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "b200fe_last_launch_count": (C.c_int64, []),

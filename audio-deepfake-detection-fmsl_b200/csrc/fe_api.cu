@@ -76,7 +76,7 @@ int pick_tt(int n_frames) {
 }
 
 int32_t common_checks(const b200fe_params* p, const void* wave, int64_t R, int64_t T, const void* tables,
-                      const void* out) {
+                      const void* out, int wave_align = 4) {
   int32_t st = fe_validate_params(p);
   if (st != B200FE_OK) return st;
   if (!wave || !tables || !out) { fe_set_error("wave / tables / out is NULL"); return B200FE_ERR_BAD_ARG; }
@@ -87,8 +87,9 @@ int32_t common_checks(const b200fe_params* p, const void* wave, int64_t R, int64
     return B200FE_ERR_BAD_ARG;
   }
   if (((uintptr_t)tables & 15) != 0) { fe_set_error("tables must be 16-byte aligned"); return B200FE_ERR_ALIGNMENT; }
-  if (((uintptr_t)wave & 3) != 0 || ((uintptr_t)out & 3) != 0) {
-    fe_set_error("wave / out must be 4-byte aligned");
+  if (((uintptr_t)wave & (wave_align - 1)) != 0 || ((uintptr_t)out & 3) != 0) {
+    if (wave_align == 4) fe_set_error("wave / out must be 4-byte aligned");
+    else fe_set_error("wave must be %d-byte and out 4-byte aligned", wave_align);
     return B200FE_ERR_ALIGNMENT;
   }
   return check_device();
@@ -121,18 +122,27 @@ static bool needs_dense_rows(const b200fe_params* p, bool ragged) {
   return p->variant == B200FE_VARIANT_DFT_GEMM && (ragged || p->preemph != 0.0f);
 }
 
-static int64_t dense_rows_bytes(const b200fe_params* p, bool ragged, int64_t chunk, int64_t T) {
-  return needs_dense_rows(p, ragged) ? ((chunk * T * 4 + 255) & ~(int64_t)255) : 0;
+// pcm16: 16-bit PCM input, which both kernel families read only as staged dense float32 rows
+static int64_t dense_rows_bytes(const b200fe_params* p, bool ragged, bool pcm16, int64_t chunk, int64_t T) {
+  return (pcm16 || needs_dense_rows(p, ragged)) ? ((chunk * T * 4 + 255) & ~(int64_t)255) : 0;
 }
 
-extern "C" int64_t b200fe_workspace_bytes_ex(const b200fe_params* p, int64_t R, int64_t T, int32_t ragged) {
+static int64_t features_workspace_bytes(const b200fe_params* p, int64_t R, int64_t T, bool ragged, bool pcm16) {
   const int64_t nf = b200fe_n_frames(p, T);
   if (nf < 0) return nf;
   if (R < 1) { fe_set_error("R=%lld must be >= 1", (long long)R); return B200FE_ERR_BAD_ARG; }
   if (p->n_filter < 1) { fe_set_error("n_filter must be >= 1 for the feature path"); return B200FE_ERR_BAD_ARG; }
   const int64_t chunk = chunk_rows_for(p, R, nf);
   return group_max_bytes(p, R) + ((fe_align16(chunk * p->n_filter * nf * 4) + 255) & ~(int64_t)255) +
-         dense_rows_bytes(p, ragged != 0, chunk, T) + fe_gemm_workspace_bytes(p, chunk, T);
+         dense_rows_bytes(p, ragged, pcm16, chunk, T) + fe_gemm_workspace_bytes(p, chunk, T);
+}
+
+extern "C" int64_t b200fe_workspace_bytes_ex(const b200fe_params* p, int64_t R, int64_t T, int32_t ragged) {
+  return features_workspace_bytes(p, R, T, ragged != 0, false);
+}
+
+extern "C" int64_t b200fe_workspace_bytes_ragged_i16(const b200fe_params* p, int64_t R, int64_t T) {
+  return features_workspace_bytes(p, R, T, true, true);
 }
 
 extern "C" int64_t b200fe_workspace_bytes(const b200fe_params* p, int64_t R, int64_t T) {
@@ -175,19 +185,22 @@ extern "C" int32_t b200fe_spectrogram_forward(const float* wave, int64_t R, int6
   return B200FE_OK;
 }
 
-static int32_t run_features(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
+// wave: float32 samples, or 16-bit PCM (pcm16: ragged only; every row is staged as dense float32 rows, x / 32768)
+static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T, const int64_t* offsets,
                             const int32_t* lengths, const b200fe_params* p, const void* tables,
                             float* out, void* workspace, size_t workspace_bytes, void* stream_,
                             bool energies_only) {
   g_launches = 0;
-  int32_t st = common_checks(p, wave, R, T, tables, out);
+  const float* wave = (const float*)wave_;
+  int32_t st = common_checks(p, wave_, R, T, tables, out, pcm16 ? 2 : 4);
   if (st != B200FE_OK) return st;
-  if ((offsets == nullptr) != (lengths == nullptr)) {
-    fe_set_error("offsets and lengths must both be given or both be NULL");
+  if ((offsets == nullptr) != (lengths == nullptr) || (pcm16 && offsets == nullptr)) {
+    fe_set_error(pcm16 ? "16-bit PCM input needs offsets and lengths"
+                       : "offsets and lengths must both be given or both be NULL");
     return B200FE_ERR_BAD_ARG;
   }
   if (p->n_filter < 1) { fe_set_error("n_filter must be >= 1 for the feature path"); return B200FE_ERR_BAD_ARG; }
-  const int64_t need = b200fe_workspace_bytes_ex(p, R, T, offsets != nullptr);
+  const int64_t need = features_workspace_bytes(p, R, T, offsets != nullptr, pcm16);
   if (need < 0) return (int32_t)need;
   if (!workspace || workspace_bytes < (size_t)need) {
     fe_set_error("workspace: %zu bytes given, %lld needed", workspace_bytes, (long long)need);
@@ -202,7 +215,8 @@ static int32_t run_features(const float* wave, int64_t R, int64_t T, const int64
       fe_set_error("variant dft_gemm does not support this configuration");
       return B200FE_ERR_UNSUPPORTED;
     }
-    if (!fe_stream_supported(p, T, R) || (!needs_dense_rows(p, offsets != nullptr) && ((uintptr_t)wave & 15) != 0)) {
+    if (!fe_stream_supported(p, T, R) ||
+        (!pcm16 && !needs_dense_rows(p, offsets != nullptr) && ((uintptr_t)wave & 15) != 0)) {
       fe_set_error("variant dft_gemm needs T %% 4 == 0, T > n_fft/2 and a 16-byte aligned waveform (TMA)");
       return B200FE_ERR_UNSUPPORTED;
     }
@@ -216,8 +230,8 @@ static int32_t run_features(const float* wave, int64_t R, int64_t T, const int64
   unsigned int* gmax = needs_group_max(p) ? (unsigned int*)workspace : nullptr;
   float* energies = (float*)((char*)workspace + group_max_bytes(p, R));
   float* dense = (float*)((char*)energies + ((fe_align16(chunk * p->n_filter * (int64_t)n_frames * 4) + 255) & ~(int64_t)255));
-  const bool staged = variant == B200FE_VARIANT_DFT_GEMM && needs_dense_rows(p, offsets != nullptr);
-  void* gemm_ws = (char*)dense + dense_rows_bytes(p, offsets != nullptr, chunk, T);
+  const bool staged = pcm16 || (variant == B200FE_VARIANT_DFT_GEMM && needs_dense_rows(p, offsets != nullptr));
+  void* gemm_ws = (char*)dense + dense_rows_bytes(p, offsets != nullptr, pcm16, chunk, T);
   const size_t row_energy_floats = (size_t)p->n_filter * n_frames;
 
   if (gmax) {
@@ -277,7 +291,29 @@ static int32_t run_features(const float* wave, int64_t R, int64_t T, const int64
     const int64_t nr = R - r0 < chunk ? R - r0 : chunk;
     cudaError_t e;
     if (energies_only) fa.out = out + (size_t)r0 * row_energy_floats;
-    if (variant == B200FE_VARIANT_DFT_GEMM) {
+    if (pcm16) {
+      // every row staged (pre-emphasis included), then read as dense rows of this chunk by either kernel family
+      e = fe_launch_dense_rows((const int16_t*)wave_, offsets, lengths, r0, nr, T, p->preemph, dense, stream);
+      if (e != cudaSuccess) return cuda_fail(e, "dense-rows kernel launch");
+      g_launches += (nr + 65534) / 65535;
+      fe_fft_args fs = fa;
+      fs.wave = nullptr;
+      fs.wave_chunk = dense;
+      fs.offsets = nullptr;
+      fs.lengths = nullptr;
+      fs.preemph = 0.0f;
+      if (variant == B200FE_VARIANT_DFT_GEMM) {
+        int launches = 0;
+        e = fe_stream_launch(p, fs, r0, nr, gemm_ws, stream, &launches);
+        if (e != cudaSuccess) return cuda_fail(e, "dft-gemm kernel launch");
+        g_launches += launches;
+      } else {
+        fs.row_base = r0;
+        e = fe_launch_fft(fs, 1, nr, stream);
+        if (e != cudaSuccess) return cuda_fail(e, "fft kernel launch");
+        ++g_launches;
+      }
+    } else if (variant == B200FE_VARIANT_DFT_GEMM) {
       int launches = 0;
       if (staged) {
         // Ragged clips that pad() only truncates (len >= T) and that start 16-byte aligned are read where they lie
@@ -337,13 +373,19 @@ static int32_t run_features(const float* wave, int64_t R, int64_t T, const int64
 extern "C" int32_t b200fe_features_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
                                            const int32_t* lengths, const b200fe_params* p, const void* tables,
                                            float* out, void* workspace, size_t workspace_bytes, void* stream) {
-  return run_features(wave, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
+  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
+}
+
+extern "C" int32_t b200fe_features_forward_ragged_i16(const int16_t* pcm, int64_t R, int64_t T, const int64_t* offsets,
+                                                      const int32_t* lengths, const b200fe_params* p, const void* tables,
+                                                      float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  return run_features(pcm, true, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
 }
 
 extern "C" int32_t b200fe_fbank_energies_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
                                                  const int32_t* lengths, const b200fe_params* p, const void* tables,
                                                  float* out, void* workspace, size_t workspace_bytes, void* stream) {
-  return run_features(wave, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, true);
+  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, true);
 }
 
 extern "C" int32_t b200fe_lfcc_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
@@ -377,82 +419,184 @@ extern "C" int32_t b200fe_compute_deltas(const float* in, int64_t rows, int64_t 
 
 // ---- host-buffer path ---------------------------------------------------------------------------
 namespace {
-struct host_slot_layout {
-  int64_t pcm_bytes, wave_bytes, out_bytes, ws_bytes, slot_bytes;
+// What the host loop streams: dense rows [R][T], or ragged clips (offsets != NULL) in a flat buffer of n_samples.
+struct host_input {
+  const void* data;
+  int32_t sample_bytes;      // 2 = 16-bit PCM (converted x / 32768 on the device), 4 = float32
+  const int64_t* offsets;    // host clip table (ragged), else NULL
+  const int32_t* lengths;
+  int64_t n_samples;
 };
-int32_t host_layout(const b200fe_params* p, int64_t chunk_rows, int64_t T, bool pcm16, host_slot_layout* L) {
+
+// Ragged chunks: the copy span of a chunk holds up to chunk_rows * (T + kSpanSlack) samples, so that chunk_rows clips of
+// at most T samples packed with up to kSpanSlack samples of alignment slack between them fit one slot.
+constexpr int64_t kSpanSlack = 16;
+
+// One slot per stream: [input | clip table | float32 rows | features | workspace of the dense forward call]
+struct host_slot_layout {
+  int64_t in_bytes, idx_bytes, wave_bytes, out_bytes, ws_bytes, slot_bytes;
+};
+
+// params of the dense forward call of a ragged chunk: pre-emphasis is applied while the rows are staged
+b200fe_params staged_params(const b200fe_params* p) {
+  b200fe_params q = *p;
+  q.preemph = 0.0f;
+  return q;
+}
+
+int32_t host_layout(const b200fe_params* p, int64_t chunk_rows, int64_t T, int32_t sample_bytes, bool ragged,
+                    host_slot_layout* L) {
   const int64_t nf = b200fe_n_frames(p, T);
   if (nf < 0) return (int32_t)nf;
   const int64_t n_out = b200fe_n_out_channels(p);
-  const int64_t ws = b200fe_workspace_bytes(p, chunk_rows, T);
+  const b200fe_params q = ragged ? staged_params(p) : *p;
+  const int64_t ws = b200fe_workspace_bytes(&q, chunk_rows, T);
   if (ws < 0) return (int32_t)ws;
-  L->pcm_bytes = pcm16 ? ((chunk_rows * T * 2 + 255) & ~(int64_t)255) : 0;
+  if (ragged) {
+    L->in_bytes = (chunk_rows * (T + kSpanSlack) * sample_bytes + 255) & ~(int64_t)255;
+    L->idx_bytes = ((chunk_rows * 8 + 255) & ~(int64_t)255) + ((chunk_rows * 4 + 255) & ~(int64_t)255);
+  } else {
+    L->in_bytes = sample_bytes == 2 ? ((chunk_rows * T * 2 + 255) & ~(int64_t)255) : 0;
+    L->idx_bytes = 0;
+  }
   L->wave_bytes = (chunk_rows * T * 4 + 255) & ~(int64_t)255;
   L->out_bytes = (chunk_rows * n_out * nf * 4 + 255) & ~(int64_t)255;
   L->ws_bytes = (ws + 255) & ~(int64_t)255;
-  L->slot_bytes = L->pcm_bytes + L->wave_bytes + L->out_bytes + L->ws_bytes;
+  L->slot_bytes = L->in_bytes + L->idx_bytes + L->wave_bytes + L->out_bytes + L->ws_bytes;
   return B200FE_OK;
 }
 
-int64_t host_staging_bytes(const b200fe_params* p, int64_t chunk_rows, int64_t T, int32_t n_streams, bool pcm16) {
+int64_t host_staging_bytes(const b200fe_params* p, int64_t chunk_rows, int64_t T, int32_t n_streams,
+                           int32_t sample_bytes, bool ragged) {
   if (chunk_rows < 1 || n_streams < 1 || n_streams > 4) {
     fe_set_error("chunk_rows=%lld n_streams=%d out of range", (long long)chunk_rows, n_streams);
     return B200FE_ERR_BAD_ARG;
   }
+  if (sample_bytes != 2 && sample_bytes != 4) {
+    fe_set_error("sample_bytes=%d must be 2 (16-bit PCM) or 4 (float32)", sample_bytes);
+    return B200FE_ERR_BAD_ARG;
+  }
   host_slot_layout L;
-  int32_t st = host_layout(p, chunk_rows, T, pcm16, &L);
+  int32_t st = host_layout(p, chunk_rows, T, sample_bytes, ragged, &L);
   if (st != B200FE_OK) return st;
   return L.slot_bytes * n_streams;
 }
 
-// wave_host: float32 rows (pcm16 == false) or int16 PCM rows (pcm16 == true: converted on the device, x / 32768)
-int32_t forward_host(const void* wave_host, bool pcm16, int64_t R, int64_t T, const b200fe_params* p,
-                     const void* tables, float* out_host, void* staging, size_t staging_bytes, int64_t chunk_rows,
-                     void* const* streams, int32_t n_streams) {
+// The checks forward_ragged's validation makes on the device, made here on the host copy of the clip table.
+int32_t check_clip_table(const host_input& in, int64_t R) {
+  for (int64_t r = 0; r < R; ++r) {
+    const int64_t off = in.offsets[r], len = in.lengths[r];
+    if (len < 1) {
+      fe_set_error("ragged input: clip %lld has %lld samples (every clip needs at least one)", (long long)r, (long long)len);
+      return B200FE_ERR_BAD_ARG;
+    }
+    if (off < 0 || off > in.n_samples - len) {
+      fe_set_error("ragged input: clip %lld (offset %lld, %lld samples) lies outside the flat buffer of %lld samples",
+                   (long long)r, (long long)off, (long long)len, (long long)in.n_samples);
+      return B200FE_ERR_BAD_ARG;
+    }
+  }
+  return B200FE_OK;
+}
+
+// Rows [r0, r0 + n) of a ragged chunk: at most max_rows rows whose copy span -- from the lowest offset to the highest
+// offset + min(length, T): pad() reads no further -- holds at most cap samples.  One row always fits (cap >= T).
+int64_t ragged_chunk(const host_input& in, int64_t r0, int64_t max_rows, int64_t T, int64_t cap, int64_t* lo,
+                     int64_t* hi) {
+  int64_t a = in.offsets[r0], b = a + (in.lengths[r0] < T ? in.lengths[r0] : T);
+  int64_t n = 1;
+  for (; n < max_rows; ++n) {
+    const int64_t o = in.offsets[r0 + n], e = o + (in.lengths[r0 + n] < T ? in.lengths[r0 + n] : T);
+    const int64_t a2 = o < a ? o : a, b2 = e > b ? e : b;
+    if (b2 - a2 > cap) break;
+    a = a2;
+    b = b2;
+  }
+  *lo = a;
+  *hi = b;
+  return n;
+}
+
+// One loop for dense rows and ragged clips; a chunk goes to stream c % n_streams and its slot:
+//   dense:  H2D rows -> (16-bit PCM: x / 32768) -> dense forward -> D2H features
+//   ragged: H2D copy span, H2D clip table slice -> stage dense rows (pad(), x / 32768, pre-emphasis) -> dense forward
+//           without pre-emphasis -> D2H features
+int32_t forward_host(const host_input& in, int64_t R, int64_t T, const b200fe_params* p, const void* tables,
+                     float* out_host, void* staging, size_t staging_bytes, int64_t chunk_rows, void* const* streams,
+                     int32_t n_streams) {
   int64_t launches = 0;
   g_launches = 0;
-  if (!wave_host || !out_host || !staging || !streams) { fe_set_error("NULL argument"); return B200FE_ERR_BAD_ARG; }
+  const bool ragged = in.offsets != nullptr;
+  if (!in.data || !out_host || !staging || !streams || !p) { fe_set_error("NULL argument"); return B200FE_ERR_BAD_ARG; }
   if (R < 1) { fe_set_error("R=%lld must be >= 1", (long long)R); return B200FE_ERR_BAD_ARG; }
-  if (p && p->top_db_group > 1 && p->log_mode == B200FE_LOG_DB && p->top_db >= 0.0f) {
+  if (p->top_db_group > 1 && p->log_mode == B200FE_LOG_DB && p->top_db >= 0.0f) {
     fe_set_error("the host-buffer path needs top_db_group == 1 (chunks are finished independently)");
     return B200FE_ERR_UNSUPPORTED;
   }
-  const int64_t need = host_staging_bytes(p, chunk_rows, T, n_streams, pcm16);
+  const int64_t need = host_staging_bytes(p, chunk_rows, T, n_streams, in.sample_bytes, ragged);
   if (need < 0) return (int32_t)need;
   if (staging_bytes < (size_t)need) {
     fe_set_error("staging: %zu bytes given, %lld needed", staging_bytes, (long long)need);
     return B200FE_ERR_WORKSPACE;
   }
   if (((uintptr_t)staging & 255) != 0) { fe_set_error("staging must be 256-byte aligned"); return B200FE_ERR_ALIGNMENT; }
+  if (ragged) {
+    int32_t st = check_clip_table(in, R);
+    if (st != B200FE_OK) return st;
+  }
   host_slot_layout L;
-  host_layout(p, chunk_rows, T, pcm16, &L);
+  host_layout(p, chunk_rows, T, in.sample_bytes, ragged, &L);
+  const b200fe_params q = ragged ? staged_params(p) : *p;
   const int64_t nf = b200fe_n_frames(p, T);
   const int64_t n_out = b200fe_n_out_channels(p);
-  const size_t in_elt = pcm16 ? 2 : 4;
+  const size_t in_elt = (size_t)in.sample_bytes;
+  const bool pcm16 = in.sample_bytes == 2;
+  const int64_t span_cap = chunk_rows * (T + kSpanSlack);
   int64_t c = 0;
-  for (int64_t r0 = 0; r0 < R; r0 += chunk_rows, ++c) {
-    const int64_t nr = R - r0 < chunk_rows ? R - r0 : chunk_rows;
+  for (int64_t r0 = 0; r0 < R; ++c) {
+    const int64_t max_rows = R - r0 < chunk_rows ? R - r0 : chunk_rows;
+    int64_t lo = 0, hi = 0;
+    const int64_t nr = ragged ? ragged_chunk(in, r0, max_rows, T, span_cap, &lo, &hi) : max_rows;
     const int s = (int)(c % n_streams);
     cudaStream_t st = (cudaStream_t)streams[s];
     char* slot = (char*)staging + (size_t)s * L.slot_bytes;
-    int16_t* d_pcm = (int16_t*)slot;
-    float* d_wave = (float*)(slot + L.pcm_bytes);
-    float* d_out = (float*)(slot + L.pcm_bytes + L.wave_bytes);
-    void* d_ws = slot + L.pcm_bytes + L.wave_bytes + L.out_bytes;
-    // one copy per chunk and direction
-    cudaError_t e = cudaMemcpyAsync(pcm16 ? (void*)d_pcm : (void*)d_wave, (const char*)wave_host + (size_t)r0 * T * in_elt,
-                                    (size_t)nr * T * in_elt, cudaMemcpyHostToDevice, st);
-    if (e != cudaSuccess) return cuda_fail(e, "H2D copy");
-    if (pcm16) {
-      e = fe_launch_i16_rows(d_pcm, d_wave, nr * T, st);
-      if (e != cudaSuccess) return cuda_fail(e, "pcm16 conversion kernel launch");
-      ++launches;
+    void* d_in = slot;
+    char* d_idx = slot + L.in_bytes;
+    float* d_wave = (float*)(d_idx + L.idx_bytes);
+    float* d_out = (float*)((char*)d_wave + L.wave_bytes);
+    void* d_ws = (char*)d_out + L.out_bytes;
+    cudaError_t e;
+    if (!ragged) {
+      // one copy per chunk and direction
+      e = cudaMemcpyAsync(pcm16 ? d_in : (void*)d_wave, (const char*)in.data + (size_t)r0 * T * in_elt,
+                          (size_t)nr * T * in_elt, cudaMemcpyHostToDevice, st);
+      if (e != cudaSuccess) return cuda_fail(e, "H2D copy");
+      if (pcm16) {
+        e = fe_launch_i16_rows((const int16_t*)d_in, d_wave, nr * T, st);
+        if (e != cudaSuccess) return cuda_fail(e, "pcm16 conversion kernel launch");
+        ++launches;
+      }
+    } else {
+      int64_t* d_off = (int64_t*)d_idx;
+      int32_t* d_len = (int32_t*)(d_idx + ((chunk_rows * 8 + 255) & ~(int64_t)255));
+      e = cudaMemcpyAsync(d_in, (const char*)in.data + (size_t)lo * in_elt, (size_t)(hi - lo) * in_elt,
+                          cudaMemcpyHostToDevice, st);
+      if (e != cudaSuccess) return cuda_fail(e, "H2D copy");
+      e = cudaMemcpyAsync(d_off, in.offsets + r0, (size_t)nr * 8, cudaMemcpyHostToDevice, st);
+      if (e != cudaSuccess) return cuda_fail(e, "H2D copy (offsets)");
+      e = cudaMemcpyAsync(d_len, in.lengths + r0, (size_t)nr * 4, cudaMemcpyHostToDevice, st);
+      if (e != cudaSuccess) return cuda_fail(e, "H2D copy (lengths)");
+      e = pcm16 ? fe_launch_dense_rows((const int16_t*)d_in, d_off, d_len, 0, nr, T, p->preemph, d_wave, st, lo)
+                : fe_launch_dense_rows((const float*)d_in, d_off, d_len, 0, nr, T, p->preemph, d_wave, st, -1, lo);
+      if (e != cudaSuccess) return cuda_fail(e, "dense-rows kernel launch");
+      launches += (nr + 65534) / 65535;
     }
-    int32_t rc = b200fe_features_forward(d_wave, nr, T, nullptr, nullptr, p, tables, d_out, d_ws, (size_t)L.ws_bytes, st);
+    int32_t rc = b200fe_features_forward(d_wave, nr, T, nullptr, nullptr, &q, tables, d_out, d_ws, (size_t)L.ws_bytes, st);
     if (rc != B200FE_OK) return rc;
     launches += g_launches;
     e = cudaMemcpyAsync(out_host + (size_t)r0 * n_out * nf, d_out, (size_t)nr * n_out * nf * 4, cudaMemcpyDeviceToHost, st);
     if (e != cudaSuccess) return cuda_fail(e, "D2H copy");
+    r0 += nr;
   }
   for (int s = 0; s < n_streams; ++s) {
     cudaError_t e = cudaStreamSynchronize((cudaStream_t)streams[s]);
@@ -461,26 +605,47 @@ int32_t forward_host(const void* wave_host, bool pcm16, int64_t R, int64_t T, co
   g_launches = launches;
   return B200FE_OK;
 }
+
+host_input dense_input(const void* rows, int32_t sample_bytes) { return host_input{rows, sample_bytes, nullptr, nullptr, 0}; }
 }  // namespace
 
 extern "C" int64_t b200fe_host_staging_bytes(const b200fe_params* p, int64_t chunk_rows, int64_t T, int32_t n_streams) {
-  return host_staging_bytes(p, chunk_rows, T, n_streams, false);
+  return host_staging_bytes(p, chunk_rows, T, n_streams, 4, false);
 }
 
 extern "C" int64_t b200fe_host_staging_bytes_i16(const b200fe_params* p, int64_t chunk_rows, int64_t T, int32_t n_streams) {
-  return host_staging_bytes(p, chunk_rows, T, n_streams, true);
+  return host_staging_bytes(p, chunk_rows, T, n_streams, 2, false);
+}
+
+extern "C" int64_t b200fe_host_staging_bytes_ragged(const b200fe_params* p, int64_t chunk_rows, int64_t T,
+                                                    int32_t sample_bytes, int32_t n_streams) {
+  return host_staging_bytes(p, chunk_rows, T, n_streams, sample_bytes, true);
 }
 
 extern "C" int32_t b200fe_features_forward_host(const float* wave_host, int64_t R, int64_t T, const b200fe_params* p,
                                                 const void* tables, float* out_host, void* staging,
                                                 size_t staging_bytes, int64_t chunk_rows, void* const* streams,
                                                 int32_t n_streams) {
-  return forward_host(wave_host, false, R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams, n_streams);
+  return forward_host(dense_input(wave_host, 4), R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams,
+                      n_streams);
 }
 
 extern "C" int32_t b200fe_features_forward_host_i16(const int16_t* pcm_host, int64_t R, int64_t T, const b200fe_params* p,
                                                     const void* tables, float* out_host, void* staging,
                                                     size_t staging_bytes, int64_t chunk_rows, void* const* streams,
                                                     int32_t n_streams) {
-  return forward_host(pcm_host, true, R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams, n_streams);
+  return forward_host(dense_input(pcm_host, 2), R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams,
+                      n_streams);
+}
+
+extern "C" int32_t b200fe_features_forward_host_ragged(const void* clips_host, int32_t sample_bytes, int64_t n_samples,
+                                                       const int64_t* offsets_host, const int32_t* lengths_host,
+                                                       int64_t R, int64_t T, const b200fe_params* p, const void* tables,
+                                                       float* out_host, void* staging, size_t staging_bytes,
+                                                       int64_t chunk_rows, void* const* streams, int32_t n_streams) {
+  g_launches = 0;
+  if (!offsets_host || !lengths_host) { fe_set_error("offsets / lengths is NULL"); return B200FE_ERR_BAD_ARG; }
+  if (n_samples < 1) { fe_set_error("n_samples=%lld must be >= 1", (long long)n_samples); return B200FE_ERR_BAD_ARG; }
+  const host_input in{clips_host, sample_bytes, offsets_host, lengths_host, n_samples};
+  return forward_host(in, R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams, n_streams);
 }

@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(kFftThreads) fe_fft_kernel(fe_fft_args a) {
       src = a.wave + a.offsets[row];
       clip_len = a.lengths[row];
     } else {
-      src = a.wave + row * a.T;
+      src = a.wave_chunk ? a.wave_chunk + row_local * a.T : a.wave + row * a.T;
       clip_len = (int)a.T;
     }
     const int seg_here = (nf_here - 1) * hop + n_fft;
@@ -412,7 +412,7 @@ __global__ void __launch_bounds__(kFftThreads, E == 16 ? 2 : 4) fe_rfft_kernel(f
       src = a.wave + a.offsets[row_b];
       clip_len = a.lengths[row_b];
     } else {
-      src = a.wave + row_b * a.T;
+      src = a.wave_chunk ? a.wave_chunk + rl * a.T : a.wave + row_b * a.T;
       clip_len = (int)a.T;
     }
     const int seg_here = (nf_b - 1) * hop + NFFT;
@@ -932,18 +932,26 @@ __global__ void fe_deltas_kernel(const float* __restrict__ in, float* __restrict
 // ------------------------------------------------------------------------------------------------
 // fe_dense_rows_kernel : clips (ragged, repeat-padded / truncated to T as pad() does, maze5.py:280-285)
 // and / or pre-emphasis -> dense rows [rows][T] the streaming tcgen05 kernel can fetch with TMA boxes.
-// One thread = four consecutive samples of one row (T % 4 == 0), one 16-byte store.
+// One thread = four consecutive samples of one row, one 16-byte store (VEC4: T % 4 == 0; otherwise four scalar stores,
+// for the FFT variant, which reads dense rows of any T).  Samples are float32 or 16-bit PCM converted as x / 32768
+// (the expression of fe_i16_rows_kernel), read one at a time: an int16 clip may start on any 2-byte boundary.
+// Row r's clip starts offsets[r] - base samples into `wave`, which then holds only the span of the flat clip buffer
+// from sample `base` on.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) fe_dense_rows_kernel(const float* __restrict__ wave,
+FE_HD float fe_sample_f32(float x) { return x; }
+FE_HD float fe_sample_f32(int16_t x) { return (1.0f / 32768.0f) * (float)x; }
+
+template <typename S, bool VEC4>
+__global__ void __launch_bounds__(256) fe_dense_rows_kernel(const S* __restrict__ wave,
                                                            const int64_t* __restrict__ offsets,
                                                            const int32_t* __restrict__ lengths, int64_t row_base,
                                                            int T, float preemph, float* __restrict__ dst,
-                                                           int64_t flat_rel) {
+                                                           int64_t flat_rel, int64_t base) {
   const int64_t row = row_base + blockIdx.y;
-  const float* src;
+  const S* src;
   int clip_len;
   if (offsets) {
-    src = wave + offsets[row];
+    src = wave + (offsets[row] - base);
     clip_len = lengths[row];
     if (fe_clip_in_place(offsets[row], clip_len, T, flat_rel)) return;   // the streaming kernel reads this clip in place
   } else {
@@ -955,16 +963,22 @@ __global__ void __launch_bounds__(256) fe_dense_rows_kernel(const float* __restr
   for (int r = (blockIdx.x * blockDim.x + threadIdx.x) * 4; r < T; r += gridDim.x * blockDim.x * 4) {
     int c = clip_len < T ? r % clip_len : r;
     float prev = 0.0f;
-    if (preemph != 0.0f && r > 0) prev = src[c == 0 ? clip_len - 1 : c - 1];
+    if (preemph != 0.0f && r > 0) prev = fe_sample_f32(src[c == 0 ? clip_len - 1 : c - 1]);
     float v[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-      const float x = src[c];
+      const float x = (VEC4 || r + i < T) ? fe_sample_f32(src[c]) : 0.0f;
       v[i] = (preemph != 0.0f && r + i > 0) ? fmaf(-preemph, prev, x) : x;
       prev = x;
       c = (c + 1 == clip_len && clip_len < T) ? 0 : c + 1;
     }
-    *reinterpret_cast<float4*>(d + r) = make_float4(v[0], v[1], v[2], v[3]);
+    if (VEC4) {
+      *reinterpret_cast<float4*>(d + r) = make_float4(v[0], v[1], v[2], v[3]);
+    } else {
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+        if (r + i < T) d[r + i] = v[i];
+    }
   }
 }
 
@@ -1301,9 +1315,10 @@ cudaError_t fe_launch_deltas(const float* in, float* out, int64_t rows, int64_t 
   return cudaSuccess;
 }
 
-cudaError_t fe_launch_dense_rows(const float* wave, const int64_t* offsets, const int32_t* lengths,
-                                 int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
-                                 cudaStream_t stream, int64_t flat_rel) {
+template <typename S>
+static cudaError_t launch_dense_rows(const S* wave, const int64_t* offsets, const int32_t* lengths, int64_t row_base,
+                                     int64_t rows, int64_t T, float preemph, float* dst, cudaStream_t stream,
+                                     int64_t flat_rel, int64_t base) {
   // CTAs per row: each thread walks its row in T / (1024 bx) steps.  One CTA per 1024 samples (64 per LFCC row) was
   // measured slowest; 16 per row is best when every row is copied (all-staged ragged step 1.30 -> 1.24 ms per 4096
   // clips, profiles/r2_ragged_inplace.txt), 8 when rows the streaming kernel reads in place are in the batch: those
@@ -1311,15 +1326,32 @@ cudaError_t fe_launch_dense_rows(const float* wave, const int64_t* offsets, cons
   unsigned bx = (unsigned)((T / 4 + 255) / 256);
   const unsigned cap = flat_rel >= 0 ? 8 : 16;
   if (bx > cap) bx = cap;
+  const bool vec4 = (T & 3) == 0;
   for (int64_t r0 = 0; r0 < rows; r0 += 65535) {
     const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
     dim3 grid(bx, (unsigned)nr);
-    fe_dense_rows_kernel<<<grid, 256, 0, stream>>>(wave, offsets, lengths, row_base + r0, (int)T, preemph,
-                                                   dst + r0 * T, flat_rel);
+    if (vec4)
+      fe_dense_rows_kernel<S, true><<<grid, 256, 0, stream>>>(wave, offsets, lengths, row_base + r0, (int)T, preemph,
+                                                              dst + r0 * T, flat_rel, base);
+    else
+      fe_dense_rows_kernel<S, false><<<grid, 256, 0, stream>>>(wave, offsets, lengths, row_base + r0, (int)T, preemph,
+                                                               dst + r0 * T, flat_rel, base);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
   }
   return cudaSuccess;
+}
+
+cudaError_t fe_launch_dense_rows(const float* wave, const int64_t* offsets, const int32_t* lengths,
+                                 int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
+                                 cudaStream_t stream, int64_t flat_rel, int64_t base) {
+  return launch_dense_rows(wave, offsets, lengths, row_base, rows, T, preemph, dst, stream, flat_rel, base);
+}
+
+cudaError_t fe_launch_dense_rows(const int16_t* wave, const int64_t* offsets, const int32_t* lengths,
+                                 int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
+                                 cudaStream_t stream, int64_t base) {
+  return launch_dense_rows(wave, offsets, lengths, row_base, rows, T, preemph, dst, stream, (int64_t)-1, base);
 }
 
 cudaError_t fe_launch_i16_rows(const int16_t* src, float* dst, int64_t n, cudaStream_t stream) {

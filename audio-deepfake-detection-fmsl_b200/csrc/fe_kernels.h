@@ -6,8 +6,8 @@
 
 struct fe_fft_args {
   const float* wave;        // dense [R][T] or flat ragged clips
-  const float* wave_chunk;  // streaming kernel only: dense rows of THIS launch ([rows][T], first row = row_base) when the
-                            // input was staged by fe_launch_dense_rows; NULL: rows are read from `wave`
+  const float* wave_chunk;  // dense rows of THIS launch ([rows][T], first row = row_base) when the input was staged by
+                            // fe_launch_dense_rows; NULL: rows are read from `wave`
   const int64_t* offsets;   // ragged: start of each row's clip (floats), else NULL
   const int32_t* lengths;   // ragged: clip lengths, else NULL
   // streaming kernel, ragged input read partly in place (in_place != 0): `wave` is then the lower of the two buffers,
@@ -68,10 +68,15 @@ cudaError_t fe_launch_cmvn(float* out, int64_t n_series, int n_frames, cudaStrea
 cudaError_t fe_launch_deltas(const float* in, float* out, int64_t rows, int64_t T, int win,
                              cudaStream_t stream);
 // Dense [rows][T] copy of rows [row_base, row_base+rows): repeat-pad / truncate ragged clips and apply
-// pre-emphasis, so the streaming kernel (TMA boxes over dense rows) serves those inputs too.  T % 4 == 0.
+// pre-emphasis, so the streaming kernel (TMA boxes over dense rows) serves those inputs too.  dst 16-byte aligned.
+// Ragged row r reads its clip at wave + offsets[r] - base (`wave` may hold only a span of the flat buffer).
 cudaError_t fe_launch_dense_rows(const float* wave, const int64_t* offsets, const int32_t* lengths,
                                  int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
-                                 cudaStream_t stream, int64_t flat_rel = -1);
+                                 cudaStream_t stream, int64_t flat_rel = -1, int64_t base = 0);
+// The same from 16-bit PCM (x / 32768, exact); every row is written (no clip is read in place).
+cudaError_t fe_launch_dense_rows(const int16_t* wave, const int64_t* offsets, const int32_t* lengths,
+                                 int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
+                                 cudaStream_t stream, int64_t base = 0);
 // 16-bit PCM -> float32 (x / 32768), n samples; src 8-byte and dst 16-byte aligned.
 cudaError_t fe_launch_i16_rows(const int16_t* src, float* dst, int64_t n, cudaStream_t stream);
 #endif

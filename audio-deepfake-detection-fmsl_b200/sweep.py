@@ -177,3 +177,65 @@ def score_host_pcm(frontend: nn.Module, scorer: nn.Module, pcm_host: Tensor, dev
     out_host.copy_(scores, non_blocking=True)
     cur.synchronize()
     return out_host
+
+
+def score_host_ragged(frontend: nn.Module, scorer: nn.Module, flat_host: Tensor, offsets: Tensor, lengths: Tensor,
+                      device: torch.device, *, max_len: int = UTT_LEN, chunk_rows: int = 1024, n_streams: int = 2,
+                      out_host: Optional[Tensor] = None) -> Tensor:
+    """``score_host_pcm`` for variable-length clips in HOST memory (maze5.py:297-351 loader and :280-285 ``pad()`` ->
+    :415-430 scoring loop): a flat int16 PCM or float32 CPU buffer (pinned for asynchronous copies) and its int64
+    ``offsets`` / int32 ``lengths`` clip table.  The table is checked once on the host; then each chunk of
+    ``chunk_rows`` rows copies the span of the flat buffer its clips occupy (up to ``max_len`` samples each: what
+    ``pad()`` reads) and its offsets rebased to that span on its own stream, and runs ``frontend.forward_ragged_pcm``
+    (int16) or ``frontend.forward_ragged`` (float32) and the classifier there.  Features stay on the device; returns
+    the bonafide scores ``float32[R]`` on the host (pinned), those of ``scorer(frontend.forward_ragged(...))`` on the
+    same chunks."""
+    if flat_host.device.type != "cpu" or flat_host.dim() != 1 or flat_host.dtype not in (torch.int16, torch.float32):
+        raise TypeError("score_host_ragged expects a 1-D int16 (16-bit PCM) or float32 CPU tensor")
+    if offsets.dtype != torch.int64 or lengths.dtype != torch.int32:
+        raise TypeError("offsets must be int64 and lengths int32")
+    off = offsets.cpu().numpy().astype(np.int64)
+    ln = lengths.cpu().numpy().astype(np.int64)
+    R = off.size
+    if ln.size != R or R < 1:
+        raise ValueError("offsets and lengths must have the same, non-zero number of entries")
+    if (ln < 1).any():
+        raise ValueError("ragged input: every clip must have at least one sample")
+    if (off < 0).any() or (off + ln > flat_host.numel()).any():
+        raise ValueError("ragged input: a clip lies outside the flat buffer")
+    T = int(max_len)
+    chunk_rows = max(1, min(int(chunk_rows), R))
+    n_streams = max(1, min(int(n_streams), 4))
+    ends = off + np.minimum(ln, T)
+    chunks = []                                   # (r0, r1, span lo, span hi)
+    for r0 in range(0, R, chunk_rows):
+        r1 = min(R, r0 + chunk_rows)
+        chunks.append((r0, r1, int(off[r0:r1].min()), int(ends[r0:r1].max())))
+    rebased = torch.from_numpy(np.concatenate([off[a:b] - lo for a, b, lo, _ in chunks])).pin_memory()
+    lengths_pinned = torch.from_numpy(ln.astype(np.int32)).pin_memory()
+    pcm16 = flat_host.dtype == torch.int16
+    span_max = [max((hi - lo for k, (_, _, lo, hi) in enumerate(chunks) if k % n_streams == s), default=1)
+                for s in range(n_streams)]
+    streams = [torch.cuda.Stream(device=device) for _ in range(n_streams)]
+    staging = [torch.empty(n, dtype=flat_host.dtype, device=device) for n in span_max]
+    scores = torch.empty(R, dtype=torch.float32, device=device)
+    cur = torch.cuda.current_stream(device)
+    for s in streams:
+        s.wait_stream(cur)
+    for c, (r0, r1, lo, hi) in enumerate(chunks):
+        s = streams[c % n_streams]
+        with torch.cuda.stream(s), torch.no_grad():
+            d = staging[c % n_streams][:hi - lo]
+            d.copy_(flat_host[lo:hi], non_blocking=True)
+            d_off = rebased[r0:r1].to(device, non_blocking=True)
+            d_len = lengths_pinned[r0:r1].to(device, non_blocking=True)
+            fwd = frontend.forward_ragged_pcm if pcm16 else frontend.forward_ragged
+            feats = fwd(d, d_off, d_len, max_len=T, validate=False)
+            scores[r0:r1] = scorer(feats)[:, 1]                       # maze5.py:425
+    for s in streams:
+        cur.wait_stream(s)
+    if out_host is None:
+        out_host = torch.empty(R, dtype=torch.float32, pin_memory=True)
+    out_host.copy_(scores, non_blocking=True)
+    cur.synchronize()
+    return out_host

@@ -246,6 +246,27 @@ class FrontEndEngine:
         if wave.device.type != "cuda":
             raise ValueError("waveform must live on a CUDA device: this front-end has no CPU path")
 
+    @staticmethod
+    def _check_ragged(flat: Tensor, offsets: Tensor, lengths: Tensor, validate: bool) -> int:
+        """The clip table of a ragged call on the device: returns its row count.  ``validate`` checks it on the device
+        (one host synchronisation; skipped during stream capture, where ``.tolist()`` cannot run)."""
+        R = offsets.numel()
+        if offsets.dtype != torch.int64 or lengths.dtype != torch.int32:
+            raise TypeError("offsets must be int64 and lengths int32")
+        if offsets.device != flat.device or lengths.device != flat.device:
+            raise ValueError("offsets / lengths must be on the waveform's device")
+        if lengths.numel() != R or R < 1:
+            raise ValueError("offsets and lengths must have the same, non-zero number of entries")
+        if validate and not torch.cuda.is_current_stream_capturing():   # (.tolist() cannot run in a capture)
+            l64 = lengths.to(torch.int64)
+            bad = torch.stack([(l64 < 1).any(), (offsets < 0).any(), ((offsets + l64) > flat.numel()).any()])
+            bad = bad.tolist()
+            if bad[0]:
+                raise ValueError("ragged input: every clip must have at least one sample")
+            if bad[1] or bad[2]:
+                raise ValueError("ragged input: a clip lies outside the flat buffer")
+        return R
+
     # -- calls -----------------------------------------------------------------------------------
     def spectrogram(self, wave2d: Tensor) -> Tensor:
         self._check_wave(wave2d)
@@ -289,21 +310,7 @@ class FrontEndEngine:
         else:
             if lengths is None or T is None:
                 raise ValueError("ragged input needs offsets, lengths and T")
-            R = offsets.numel()
-            if offsets.dtype != torch.int64 or lengths.dtype != torch.int32:
-                raise TypeError("offsets must be int64 and lengths int32")
-            if offsets.device != dev or lengths.device != dev:
-                raise ValueError("offsets / lengths must be on the waveform's device")
-            if lengths.numel() != R or R < 1:
-                raise ValueError("offsets and lengths must have the same, non-zero number of entries")
-            if validate and not torch.cuda.is_current_stream_capturing():   # (.tolist() cannot run in a capture)
-                l64 = lengths.to(torch.int64)
-                bad = torch.stack([(l64 < 1).any(), (offsets < 0).any(), ((offsets + l64) > wave2d.numel()).any()])
-                bad = bad.tolist()
-                if bad[0]:
-                    raise ValueError("ragged input: every clip must have at least one sample")
-                if bad[1] or bad[2]:
-                    raise ValueError("ragged input: a clip lies outside the flat buffer")
+            R = self._check_ragged(wave2d, offsets, lengths, validate)
         p = self._params_for_call(self._params_with_group(group), T, wave2d.data_ptr(), offsets is not None)
         nf = self.n_frames(T)
         if out is None:
@@ -329,6 +336,38 @@ class FrontEndEngine:
         else:
             with torch.cuda.device(dev):
                 launch()
+        return out
+
+    def features_ragged_pcm(self, flat_i16: Tensor, offsets: Tensor, lengths: Tensor, T: int,
+                            out: Optional[Tensor] = None, validate: bool = True) -> Tensor:
+        """The ragged call of ``features`` with 16-bit PCM clips on the device (``b200fe_features_forward_ragged_i16``):
+        every row is staged as a dense float32 row, ``x / 32768`` (exact), so the features are those of the float32
+        ragged call on ``flat_i16.float() / 32768``, bit for bit.  Returns ``(R, n_out, n_frames)``."""
+        if not isinstance(flat_i16, Tensor) or flat_i16.dtype != torch.int16:
+            raise TypeError(f"features_ragged_pcm expects int16 PCM, got "
+                            f"{flat_i16.dtype if isinstance(flat_i16, Tensor) else type(flat_i16)}")
+        if flat_i16.device.type != "cuda":
+            raise ValueError("waveform must live on a CUDA device: this front-end has no CPU path")
+        if not flat_i16.is_contiguous():
+            raise ValueError("the flat clip buffer must be contiguous")
+        dev = flat_i16.device
+        R = self._check_ragged(flat_i16, offsets, lengths, validate)
+        T = int(T)
+        p = self._params_for_call(self.params, T, None, True)
+        nf = self.n_frames(T)
+        if out is None:
+            out = torch.empty((R, self.n_out, nf), dtype=torch.float32, device=dev)
+        wkey = (R, T, "pcm16", p.variant, p.top_db_group)
+        wc = self.__dict__.setdefault("_ws_bytes_cache", {})
+        ws_bytes = wc.get(wkey)
+        if ws_bytes is None:
+            ws_bytes = wc[wkey] = _lib.check(self.lib.b200fe_workspace_bytes_ragged_i16(C.byref(p), R, T))
+        with torch.cuda.device(dev), self._lock:
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            ws = self.workspace_on(dev, ws_bytes, stream)
+            _lib.check(self.lib.b200fe_features_forward_ragged_i16(
+                flat_i16.data_ptr(), R, T, offsets.data_ptr(), lengths.data_ptr(), C.byref(p),
+                self.tables_on(dev).data_ptr(), out.data_ptr(), ws.data_ptr(), ws.numel(), C.c_void_p(stream)))
         return out
 
     def fbank_energies(self, wave2d: Tensor, out: Optional[Tensor] = None) -> Tensor:
@@ -370,6 +409,15 @@ class FrontEndEngine:
         p = self._params_for_call(self.params, T, None, False)   # staged rows are 256-byte aligned
         sizer = self.lib.b200fe_host_staging_bytes_i16 if pcm16 else self.lib.b200fe_host_staging_bytes
         need = _lib.check(sizer(C.byref(p), chunk_rows, T, n_streams))
+        call = self.lib.b200fe_features_forward_host_i16 if pcm16 else self.lib.b200fe_features_forward_host
+        self._host_call(device, need, n_streams, lambda tables, st, arr: call(
+            wave_host.data_ptr(), R, T, C.byref(p), tables.data_ptr(), out_host.data_ptr(),
+            st.data_ptr(), st.numel(), chunk_rows, arr, n_streams))
+        return out_host
+
+    def _host_call(self, device: torch.device, need: int, n_streams: int, call) -> None:
+        """Runs ``call(tables, staging, streams)`` under ``_host_lock`` with the engine's host staging (grown to ``need``
+        bytes) and its copy streams, shared by every host-buffer call on ``device``."""
         with self._host_lock:
             st, streams = self._host_staging.get(device, (None, None))
             if st is None or st.numel() < need:
@@ -381,10 +429,48 @@ class FrontEndEngine:
             with torch.cuda.device(device):
                 tables = self.tables_on(device)
                 torch.cuda.current_stream(device).synchronize()  # tables upload finished
-                call = self.lib.b200fe_features_forward_host_i16 if pcm16 else self.lib.b200fe_features_forward_host
-                _lib.check(call(
-                    wave_host.data_ptr(), R, T, C.byref(p), tables.data_ptr(), out_host.data_ptr(),
-                    st.data_ptr(), st.numel(), chunk_rows, arr, n_streams))
+                _lib.check(call(tables, st, arr))
+
+    def features_host_ragged(self, flat_host: Tensor, offsets_host: Tensor, lengths_host: Tensor, T: int,
+                             out_host: Optional[Tensor] = None, *, device=None, chunk_rows: int = 512,
+                             n_streams: int = 3) -> Tensor:
+        """End-to-end path for variable-length clips in HOST memory (``b200fe_features_forward_host_ragged``): a flat
+        float32 or int16 PCM CPU buffer (ideally pinned) with an int64 ``offsets`` / int32 ``lengths`` clip table in,
+        HOST features ``(R, n_out, n_frames)`` out, each clip repeat-padded / truncated to ``T`` as ``pad()`` does.
+        Only the samples ``pad()`` reads of each chunk's span cross PCIe (pack with ``pack_clips(max_len=T)`` to keep
+        the spans tight); the rows are staged on the device.  The clip table is checked on the host (``ValueError``).
+        Features are those of ``features`` / ``features_ragged_pcm`` on the same clips, bit for bit.  Shares the staging
+        buffer, copy streams and lock of ``features_host``."""
+        if not isinstance(flat_host, Tensor) or flat_host.device.type != "cpu" or flat_host.dim() != 1 \
+                or flat_host.dtype not in (torch.float32, torch.int16):
+            raise TypeError("features_host_ragged expects a 1-D float32 (or int16 PCM) CPU tensor")
+        if not isinstance(offsets_host, Tensor) or not isinstance(lengths_host, Tensor) \
+                or offsets_host.dtype != torch.int64 or lengths_host.dtype != torch.int32:
+            raise TypeError("offsets must be int64 and lengths int32")
+        if offsets_host.device.type != "cpu" or lengths_host.device.type != "cpu":
+            raise ValueError("offsets / lengths must be CPU tensors")
+        R = offsets_host.numel()
+        if lengths_host.numel() != R or R < 1:
+            raise ValueError("offsets and lengths must have the same, non-zero number of entries")
+        if flat_host.numel() < 1:
+            raise ValueError("the flat clip buffer is empty")
+        flat_host = flat_host.contiguous()
+        offsets_host = offsets_host.contiguous()
+        lengths_host = lengths_host.contiguous()
+        sample_bytes = flat_host.element_size()
+        T = int(T)
+        device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        nf = self.n_frames(T)
+        if out_host is None:
+            out_host = torch.empty((R, self.n_out, nf), dtype=torch.float32, pin_memory=True)
+        chunk_rows = max(1, min(int(chunk_rows), R))
+        n_streams = max(1, min(int(n_streams), 4))
+        p = self._params_for_call(self.params, T, None, True)   # every row is staged (256-byte aligned)
+        need = _lib.check(self.lib.b200fe_host_staging_bytes_ragged(C.byref(p), chunk_rows, T, sample_bytes, n_streams))
+        self._host_call(device, need, n_streams, lambda tables, st, arr: self.lib.b200fe_features_forward_host_ragged(
+            flat_host.data_ptr(), sample_bytes, flat_host.numel(), offsets_host.data_ptr(), lengths_host.data_ptr(),
+            R, T, C.byref(p), tables.data_ptr(), out_host.data_ptr(), st.data_ptr(), st.numel(), chunk_rows, arr,
+            n_streams))
         return out_host
 
 
@@ -398,15 +484,35 @@ def _pack_rows(waveform: Tensor) -> Tuple[Tensor, Tuple[int, ...]]:
     return w, shape
 
 
-def pack_clips(clips, align: int = 4, pin_memory: bool = False) -> Tuple[Tensor, Tensor, Tensor]:
+def pack_clips(clips, align: int = 4, pin_memory: bool = False, *, dtype: torch.dtype = torch.float32,
+               max_len: Optional[int] = None) -> Tuple[Tensor, Tensor, Tensor]:
     """Variable-length clips (1-D float32 tensors or arrays, as the reference's loader reads them before ``pad()``,
     maze5.py:280-351) -> the ragged input of ``forward_ragged``: ``(flat, offsets int64, lengths int32)`` on the
     host.  Every clip starts on a multiple of ``align`` samples (default 4 = 16 bytes, up to 3 zero samples of slack
     between clips): clips that ``pad()`` only truncates are then read by the streaming kernel where they lie instead
-    of being staged as dense rows.  An empty clip raises, as ``pad()`` does."""
+    of being staged as dense rows.  An empty clip raises, as ``pad()`` does.
+
+    ``dtype=torch.int16`` packs 16-bit PCM clips bit for bit (for ``forward_ragged_pcm`` / ``forward_host_ragged``);
+    every clip must then be int16 already (``TypeError`` otherwise: no implicit quantisation).  ``max_len`` keeps only
+    the first ``max_len`` samples of each clip and records the truncated length: ``pad(clip, T) == pad(clip[:T], T)``,
+    so the features are unchanged for ``T <= max_len``, and the buffer holds only samples ``pad()`` reads."""
     if align < 1:
         raise ValueError("align must be >= 1")
-    ts = [torch.as_tensor(c, dtype=torch.float32).reshape(-1) for c in clips]
+    if dtype not in (torch.float32, torch.int16):
+        raise ValueError(f"dtype must be torch.float32 or torch.int16, got {dtype}")
+    if max_len is not None and int(max_len) < 1:
+        raise ValueError("max_len must be >= 1")
+    if dtype == torch.int16:
+        ts = []
+        for i, c in enumerate(clips):
+            t = torch.as_tensor(c)
+            if t.dtype != torch.int16:
+                raise TypeError(f"clip {i} is {t.dtype}: pack_clips(dtype=torch.int16) takes int16 PCM clips only")
+            ts.append(t.reshape(-1))
+    else:
+        ts = [torch.as_tensor(c, dtype=torch.float32).reshape(-1) for c in clips]
+    if max_len is not None:
+        ts = [t[:int(max_len)] for t in ts]
     if not ts:
         raise ValueError("no clips")
     lengths = torch.tensor([t.numel() for t in ts], dtype=torch.int64)
@@ -414,7 +520,7 @@ def pack_clips(clips, align: int = 4, pin_memory: bool = False) -> Tuple[Tensor,
         raise ValueError("every clip must have at least one sample")
     slots = (lengths + align - 1) // align * align
     offsets = torch.cumsum(slots, 0) - slots
-    flat = torch.zeros(int(slots.sum()), dtype=torch.float32, pin_memory=pin_memory)
+    flat = torch.zeros(int(slots.sum()), dtype=dtype, pin_memory=pin_memory)
     for t, o in zip(ts, offsets.tolist()):
         flat[o:o + t.numel()] = t
     return flat, offsets, lengths.to(torch.int32)
@@ -473,9 +579,21 @@ class _Base(nn.Module):
         inside the loader exactly like ``pad()`` (maze5.py:280-285).  Returns ``(R, C, n_frames)``."""
         return self.engine.features(flat, group=1, offsets=offsets, lengths=lengths, T=int(max_len), validate=validate)
 
+    def forward_ragged_pcm(self, flat: Tensor, offsets: Tensor, lengths: Tensor, max_len: int = 64600,
+                           validate: bool = True) -> Tensor:
+        """``forward_ragged`` for 16-bit PCM clips on the device (``flat`` int16, converted ``x / 32768`` while the rows
+        are staged): the features of ``forward_ragged(flat.float() / 32768, ...)``, bit for bit."""
+        return self.engine.features_ragged_pcm(flat, offsets, lengths, int(max_len), validate=validate)
+
     def forward_host(self, wave_host: Tensor, out_host: Optional[Tensor] = None, **kw) -> Tensor:
         """Host in / host out with pipelined copies (see ``FrontEndEngine.features_host``)."""
         return self.engine.features_host(wave_host, out_host, **kw)
+
+    def forward_host_ragged(self, flat_host: Tensor, offsets: Tensor, lengths: Tensor, max_len: int = 64600,
+                            out_host: Optional[Tensor] = None, **kw) -> Tensor:
+        """Variable-length clips (float32 or int16 PCM) in HOST memory, pad()ded to ``max_len`` on the device, HOST
+        features out (see ``FrontEndEngine.features_host_ragged``)."""
+        return self.engine.features_host_ragged(flat_host, offsets, lengths, int(max_len), out_host, **kw)
 
 
 class Spectrogram(nn.Module):

@@ -127,6 +127,18 @@ int64_t b200fe_workspace_bytes(const b200fe_params* p, int64_t R, int64_t T);
  * workspace size does not depend on how many there are). */
 int64_t b200fe_workspace_bytes_ex(const b200fe_params* p, int64_t R, int64_t T, int32_t ragged);
 
+/* The ragged call of b200fe_features_forward with 16-bit PCM clips, what the reference's loader decodes before it turns
+ * them into float32 and pad()s them (maze5.py:297-351, :280-285): every row is staged as a dense float32 row in the
+ * workspace -- repeat-padded / truncated to T, converted x / 32768 (exact), pre-emphasis applied -- for either kernel
+ * family, so the features are bit-identical to the float32 ragged call on the converted samples.
+ *   pcm  int16 device flat clips, 2-byte aligned (a clip may start on any sample);  offsets / lengths as above (required)
+ *   workspace  >= b200fe_workspace_bytes_ragged_i16(p, R, T): the ragged workspace plus one chunk of dense rows for
+ *   either variant */
+int64_t b200fe_workspace_bytes_ragged_i16(const b200fe_params* p, int64_t R, int64_t T);
+int32_t b200fe_features_forward_ragged_i16(const int16_t* pcm, int64_t R, int64_t T, const int64_t* offsets,
+                                           const int32_t* lengths, const b200fe_params* p, const void* tables,
+                                           float* out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Replaces Spectrogram.forward (transforms/_transforms.py:25; functional.py:119-145, power=2):
  *   wave  float32 device [R][T] contiguous           out  float32 device [R][n_fft/2+1][n_frames]   */
 int32_t b200fe_spectrogram_forward(const float* wave, int64_t R, int64_t T, const b200fe_params* p,
@@ -189,6 +201,27 @@ int32_t b200fe_features_forward_host_i16(const int16_t* pcm_host, int64_t R, int
                                          const void* tables, float* out_host, void* staging,
                                          size_t staging_bytes, int64_t chunk_rows, void* const* streams,
                                          int32_t n_streams);
+
+/* Variable-length clips in HOST memory: replaces the reference's loader + pad() + batching (maze5.py:297-351,
+ * :280-285) in front of the feature slot of its scoring loop (maze5.py:415-430).  Clip r is
+ * clips_host[offsets_host[r] .. + lengths_host[r]) of a flat buffer of n_samples samples, int16 PCM (sample_bytes 2,
+ * x / 32768) or float32 (sample_bytes 4); out_host float32 [R][n_out_channels][n_frames] as above.
+ * Chunks of at most chunk_rows consecutive rows are pipelined as in b200fe_features_forward_host.  A chunk copies one
+ * span of the flat buffer, from its lowest offset to its highest offset + min(length, T) (pad() reads no further), and
+ * closes early when the next row would take the span past chunk_rows * (T + 16) samples; then the chunk's slice of
+ * the clip table is copied, a kernel stages the rows dense (pad(), x / 32768, pre-emphasis) and the dense forward call
+ * runs.  Features are bit-identical to b200fe_features_forward(_ragged_i16) on the same clips.  The clip table is
+ * checked on the host before any CUDA call (every length >= 1, offset >= 0, offset + length <= n_samples:
+ * B200FE_ERR_BAD_ARG naming the first bad row).  Needs top_db_group == 1.
+ *   staging  >= b200fe_host_staging_bytes_ragged(p, chunk_rows, T, sample_bytes, n_streams), 256-byte aligned
+ *   streams  array of n_streams cudaStream_t (as void*), 1..4                                                      */
+int64_t b200fe_host_staging_bytes_ragged(const b200fe_params* p, int64_t chunk_rows, int64_t T,
+                                         int32_t sample_bytes, int32_t n_streams);
+int32_t b200fe_features_forward_host_ragged(const void* clips_host, int32_t sample_bytes, int64_t n_samples,
+                                            const int64_t* offsets_host, const int32_t* lengths_host, int64_t R,
+                                            int64_t T, const b200fe_params* p, const void* tables, float* out_host,
+                                            void* staging, size_t staging_bytes, int64_t chunk_rows,
+                                            void* const* streams, int32_t n_streams);
 
 /* ---- scoring tail on the device (SURVEY 8f-2) ---------------------------------------------------
  * Replaces the host-side  fpr, tpr, thr = sklearn.metrics.roc_curve(y, s); fnr = 1 - tpr;
