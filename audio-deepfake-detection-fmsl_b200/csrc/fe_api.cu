@@ -215,9 +215,12 @@ static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T,
       fe_set_error("variant dft_gemm does not support this configuration");
       return B200FE_ERR_UNSUPPORTED;
     }
-    if (!fe_stream_supported(p, T, R) ||
-        (!pcm16 && !needs_dense_rows(p, offsets != nullptr) && ((uintptr_t)wave & 15) != 0)) {
-      fe_set_error("variant dft_gemm needs T %% 4 == 0, T > n_fft/2 and a 16-byte aligned waveform (TMA)");
+    if (!fe_stream_supported(p, T)) {
+      fe_set_error("variant dft_gemm needs T %% 4 == 0 and T > n_fft/2 (T=%lld, n_fft=%d)", (long long)T, p->n_fft);
+      return B200FE_ERR_UNSUPPORTED;
+    }
+    if (!pcm16 && !needs_dense_rows(p, offsets != nullptr) && ((uintptr_t)wave & 15) != 0) {
+      fe_set_error("variant dft_gemm needs a 16-byte aligned waveform (TMA)");
       return B200FE_ERR_UNSUPPORTED;
     }
     variant = B200FE_VARIANT_DFT_GEMM;

@@ -79,13 +79,13 @@ __global__ void __launch_bounds__(kThreads, 1) fe_eer_kernel(const float* __rest
   const unsigned int lo = min(n, tid * per), hi = min(n, lo + per);
 
   // ---- records ------------------------------------------------------------------------------------
-  bool nan_here = false;
+  bool nonfinite_here = false;
   for (unsigned int i = tid; i < n; i += kThreads) {
     const float sc = scores[i];
-    nan_here |= sc != sc;
+    nonfinite_here |= !isfinite(sc);
     ws.rec[0][i] = ((unsigned long long)score_key(sc) << 32) | (unsigned long long)(labels[i] == 1 ? 1u : 0u);
   }
-  if (__syncthreads_or(nan_here)) {   // scikit-learn's roc_curve raises on NaN scores; here: status 2, nothing computed
+  if (__syncthreads_or(nonfinite_here)) {   // scikit-learn's roc_curve raises on NaN and infinite scores; here: status 2
     if (tid == 0) { out[0] = out[1] = out[2] = 0.0; out[3] = 2.0; }
     return;
   }

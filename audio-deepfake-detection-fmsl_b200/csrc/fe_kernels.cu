@@ -1004,7 +1004,7 @@ __global__ void __launch_bounds__(256) fe_i16_rows_kernel(const int16_t* __restr
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) fe_tail_pointwise_kernel(fe_tail_args a) {
   const int64_t row_local = blockIdx.y, row = a.row_base + row_local;
-  const int per_row = a.n_filter * a.n_frames;
+  const int64_t per_row = (int64_t)a.n_filter * a.n_frames;
   float floor_db = -INFINITY;
   if (a.log_mode == B200FE_LOG_DB && a.top_db >= 0.0f) {
     const float gmax = __uint_as_float(a.group_max[row / a.top_db_group]);
@@ -1012,7 +1012,7 @@ __global__ void __launch_bounds__(256) fe_tail_pointwise_kernel(fe_tail_args a) 
   }
   const float* src = a.energies + (size_t)row_local * per_row;
   float* dst = a.out + (size_t)row * per_row;
-  const int i0 = blockIdx.x * 1024 + threadIdx.x;
+  const int64_t i0 = (int64_t)blockIdx.x * 1024 + threadIdx.x;
   float v[4];
 #pragma unroll
   for (int u = 0; u < 4; ++u) v[u] = (i0 + 256 * u < per_row) ? src[i0 + 256 * u] : 1.0f;
@@ -1262,7 +1262,7 @@ static cudaError_t launch_tail_fast(const fe_tail_args& a_in, int64_t rows, cuda
 
 cudaError_t fe_launch_tail(const fe_tail_args& a, int64_t rows, cudaStream_t stream) {
   if (a.n_coef == 0 && a.deltas == 0 && a.force_generic != 1) {
-    const int per_row = a.n_filter * a.n_frames;
+    const int64_t per_row = (int64_t)a.n_filter * a.n_frames;
     for (int64_t r0 = 0; r0 < rows; r0 += 65535) {
       fe_tail_args b = a;
       const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;

@@ -228,8 +228,8 @@ __device__ __forceinline__ void scout_tile_global(const stream_args& a, int nF, 
 __device__ __forceinline__ void quarter_bar(int quarter) { asm volatile("bar.sync %0, 128;" ::"r"(2 + quarter) : "memory"); }   // the frame quarter's four walkers
 __device__ __forceinline__ void runs_bar(int quarter) { asm volatile("bar.sync %0, 64;" ::"r"(6 + quarter) : "memory"); }      // its two half-1 walkers
 
-// a finished filter segment of the drain: final energy of (frame, filter) -> workspace (32-bit element offsets: a
-// launch's energies are < 2^31 bytes, fe_stream_supported)
+// a finished filter segment of the drain: final energy of (frame, filter) -> workspace (32-bit element offsets:
+// fe_stream_launch keeps a launch's energies below 2^31 elements)
 struct emit_store {
   float* base;        // energies of the launch
   uint32_t off;       // (row * n_filter) * n_frames + t
@@ -742,17 +742,17 @@ int64_t fe_gemm_workspace_bytes(const b200fe_params* p, int64_t chunk_rows, int6
   return 65536;  // error flag (+ trace buffer in FE_GEMM_TRACE builds)
 }
 
-bool fe_stream_supported(const b200fe_params* p, int64_t T, int64_t rows) {
+bool fe_stream_supported(const b200fe_params* p, int64_t T) {
   if (!fe_gemm_supported(p)) return false;
-  const int64_t nF = 1 + T / p->hop_length;
-  if (nF < 2 || rows * nF >= (int64_t)1 << 30 || rows * nF * p->n_filter >= (int64_t)1 << 31) return false;   // 32-bit element offsets
-  if (T <= p->n_fft / 2 || (T & 3) != 0) return false;
-  return true;
+  return (T & 3) == 0 && T > p->n_fft / 2 && 1 + T / p->hop_length >= 2;
 }
 
-cudaError_t fe_stream_launch(const b200fe_params* p, const fe_fft_args& fa, int64_t row_base, int64_t rows,
-                             void* gemm_ws, cudaStream_t stream, int* launches) {
-  *launches = 0;
+namespace {
+
+// One launch of the streaming kernel over rows [row_base, row_base + rows) of the call, which keep the launch's frame
+// and element indices within 32 bits (fe_stream_launch).
+cudaError_t stream_launch_one(const b200fe_params* p, const fe_fft_args& fa, int64_t row_base, int64_t rows,
+                              void* gemm_ws, cudaStream_t stream) {
   stream_args a;
   const bool in_place = fa.in_place != 0 && fa.wave_chunk && fa.offsets && fa.lengths;
   a.wave = in_place ? fa.wave : (fa.wave_chunk ? fa.wave_chunk : fa.wave + row_base * fa.T);
@@ -849,6 +849,29 @@ cudaError_t fe_stream_launch(const b200fe_params* p, const fe_fft_args& fa, int6
 #endif
   if (e != cudaSuccess) return e;
   fe_stream_kernel<<<grid, kThreads, smem, stream>>>(*maps_p, a);
-  *launches = 1;
   return cudaGetLastError();
+}
+
+}  // namespace
+
+cudaError_t fe_stream_launch(const b200fe_params* p, const fe_fft_args& fa, int64_t row_base, int64_t rows,
+                             void* gemm_ws, cudaStream_t stream, int* launches) {
+  *launches = 0;
+  // The kernel indexes a launch's frames (fe_tile_geometry: frames plus one hop block per row) and energy elements
+  // (emit_store) in 32 bits: rows * n_frames < 2^30 and rows * n_filter * n_frames < 2^31 per launch.  One row always
+  // fits (T < 2^30, hop >= 32, n_filter <= 32).
+  const int64_t nF = fa.n_frames, per_row = (int64_t)p->n_filter * nF;
+  const int64_t frame_rows = (((int64_t)1 << 30) - 1) / nF, energy_rows = (((int64_t)1 << 31) - 1) / per_row;
+  const int64_t max_rows = frame_rows < energy_rows ? frame_rows : energy_rows;
+  for (int64_t r0 = 0; r0 < rows; r0 += max_rows) {
+    const int64_t nr = rows - r0 < max_rows ? rows - r0 : max_rows;
+    fe_fft_args f = fa;
+    f.out = fa.out + r0 * per_row;
+    if (fa.wave_chunk) f.wave_chunk = fa.wave_chunk + r0 * fa.T;
+    f.dense_rel = fa.dense_rel + r0 * fa.T;
+    cudaError_t e = stream_launch_one(p, f, row_base + r0, nr, gemm_ws, stream);
+    if (e != cudaSuccess) return e;
+    ++*launches;
+  }
+  return cudaSuccess;
 }

@@ -45,6 +45,8 @@ def _roc_curve(y_true: np.ndarray, y_score: np.ndarray):
     # sklearn.metrics.roc_curve(drop_intermediate=True), the call at Maze5_eval.py:588
     y_true = np.asarray(y_true) == 1
     y_score = np.asarray(y_score, dtype=np.float64)
+    if not np.isfinite(y_score).all():   # scikit-learn's check_array raises on such input
+        raise ValueError("scores contain NaN or infinite values (scikit-learn's roc_curve raises on such input too)")
     order = np.argsort(y_score, kind="mergesort")[::-1]
     y_score, y_true = y_score[order], y_true[order]
     idx = np.r_[np.where(np.diff(y_score))[0], y_true.size - 1]
@@ -99,7 +101,7 @@ def eer_min_dcf_device(y_true: torch.Tensor, y_score: torch.Tensor, *, sync: boo
         return out
     eer, dcf, thr, status = out.tolist()
     if status == 2.0:
-        raise ValueError("scores contain NaN (scikit-learn's roc_curve raises on such input too)")
+        raise ValueError("scores contain NaN or infinite values (scikit-learn's roc_curve raises on such input too)")
     if status != 0.0:
         raise ValueError("EER needs both classes present (Maze5_eval.py:577-582 returns {} in that case)")
     return eer, dcf, thr

@@ -129,7 +129,7 @@ def run_sweep(frontend: nn.Module, scorer: nn.Module, device: torch.device, *, n
     e1.record()
     eer, dcf, thr, status = metrics_dev.tolist()           # the sweep's only device -> host read of results: 32 bytes
     if status != 0.0:
-        raise ValueError("scores contain NaN" if status == 2.0 else "EER needs both classes present")
+        raise ValueError("scores contain NaN or infinite values" if status == 2.0 else "EER needs both classes present")
     eer_ms = e0.elapsed_time(e1)
     wall = time.perf_counter() - t0
     # (kept for the record and the tests: the host restatement of the reference's sklearn call on the same scores)

@@ -231,8 +231,8 @@ int32_t b200fe_features_forward_host_ragged(const void* clips_host, int32_t samp
  *   scores  float32 device [n]   per-utterance scores (maze5.py:425: log-softmax column 1)
  *   labels  int32 device [n]     1 = bonafide (positive class), anything else = spoof
  *   out4    float64 device [4]   eer, min_dcf, eer threshold, status (0 ok, 1 = only one class present: the
- *                                reference returns no metrics then, Maze5_eval.py:577-582; 2 = a score is NaN:
- *                                scikit-learn's roc_curve raises on such input)
+ *                                reference returns no metrics then, Maze5_eval.py:577-582; 2 = a score is NaN or
+ *                                infinite: scikit-learn's roc_curve raises on such input)
  *   workspace  device scratch >= b200fe_eer_workspace_bytes(n), 16-byte aligned
  * One kernel on `stream`; no synchronisation (the caller reads out4 when it needs the numbers). */
 int64_t b200fe_eer_workspace_bytes(int64_t n);

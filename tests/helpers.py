@@ -126,3 +126,27 @@ def emulate_gemm_energies(module, x):
                                          eng._blob_host.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p))
     assert rc == 0, "tables do not carry the DFT-GEMM variant"
     return out
+
+
+def eer_from_counts(values, pos, neg):
+    """``(eer, min_dcf, eer_threshold)`` of scores given as distinct float32 ``values`` with ``pos`` / ``neg`` records
+    of each, computed exactly in float64: scikit-learn's ``roc_curve`` (one point per distinct score, in decreasing
+    order; ``drop_intermediate``; a leading (0, 0, inf) point) and the reference's formulas, as
+    ``evaluation._roc_curve`` has them.  Values that compare equal (-0.0 and +0.0) form one point."""
+    v = np.asarray(values, np.float64)
+    pos, neg = np.asarray(pos, np.int64), np.asarray(neg, np.int64)
+    u, inv = np.unique(v, return_inverse=True)          # -0.0 == +0.0: one entry
+    p = np.bincount(inv, weights=pos, minlength=u.size)[::-1]
+    n = np.bincount(inv, weights=neg, minlength=u.size)[::-1]
+    thr = u[::-1]
+    present = (p + n) > 0
+    p, n, thr = p[present], n[present], thr[present]
+    tps, fps = np.cumsum(p), np.cumsum(n)               # exact: integers below 2^53
+    if len(fps) > 2:
+        keep = np.where(np.r_[True, np.logical_or(np.diff(fps, 2), np.diff(tps, 2)), True])[0]
+        fps, tps, thr = fps[keep], tps[keep], thr[keep]
+    tps, fps, thr = np.r_[0, tps], np.r_[0, fps], np.r_[np.inf, thr]
+    fpr, tpr = fps / fps[-1], tps / tps[-1]
+    fnr = 1 - tpr
+    i = int(np.nanargmin(np.absolute(fnr - fpr)))
+    return float(fpr[i]), float(np.min(fnr + fpr)), float(thr[i])

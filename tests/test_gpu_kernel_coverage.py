@@ -48,20 +48,24 @@ def gamma(n):
 
 
 # ---- float64 references --------------------------------------------------------------------------------------------
-def power_spec64(x, case):
-    """|rfft|^2 of reflect-padded frames, window centred like torch.stft: (R, n_freq, n_frames) float64."""
+def power_spec64(x, case, frames=None, first=0, T=None):
+    """|rfft|^2 of reflect-padded frames, window centred like torch.stft: (R, n_freq, n_frames) float64.
+    ``x`` holds samples [first, first + x.shape[1]) of rows of T samples (default: whole rows); ``frames`` selects
+    the frame indices to evaluate (default: all 1 + T // hop of them)."""
     n_fft, hop = case.n_fft, case.hop
+    T = x.shape[1] if T is None else T
     w = np.zeros(n_fft)
     left = (n_fft - case.win) // 2
     w[left:left + case.win] = window_of(case).double().numpy()
-    xp = np.pad(np.asarray(x, np.float64), ((0, 0), (n_fft // 2, n_fft // 2)), mode="reflect")
-    nF = 1 + x.shape[1] // hop
-    idx = np.arange(n_fft)[None, :] + hop * np.arange(nF)[:, None]
-    return (np.abs(np.fft.rfft(xp[:, idx] * w, axis=-1)) ** 2).transpose(0, 2, 1)
+    frames = np.arange(1 + T // hop) if frames is None else np.asarray(frames, np.int64)
+    idx = np.abs(np.arange(n_fft)[None, :] + hop * frames[:, None] - n_fft // 2)   # reflect about sample 0 ...
+    idx = np.where(idx >= T, 2 * (T - 1) - idx, idx) - first                        # ... and about sample T - 1
+    assert idx.min() >= 0 and idx.max() < x.shape[1], "the frames read samples outside x"
+    return (np.abs(np.fft.rfft(np.asarray(x, np.float64)[:, idx] * w, axis=-1)) ** 2).transpose(0, 2, 1)
 
 
-def energies64(x, case):
-    return np.einsum("rkt,kf->rft", power_spec64(x, case), fbank_of(case).double().numpy())
+def energies64(x, case, **window):
+    return np.einsum("rkt,kf->rft", power_spec64(x, case, **window), fbank_of(case).double().numpy())
 
 
 def stage_ratio(got, ref):
@@ -89,17 +93,20 @@ def _ulp32(v):
     return np.spacing(np.abs(v).astype(np.float32)).astype(np.float64)
 
 
-def tail64(E32, case, group):
+def tail64(E32, case, group, gmax=None):
     """Float64 tail on the device's energies, with an elementwise rounding-error bound for the float32 kernels.
     Next to each value the same linear maps are applied to absolute values (A): a sum of n float32 products is off by
-    at most gamma(n) * sum |w| |x| plus the propagated bounds of its inputs."""
+    at most gamma(n) * sum |w| |x| plus the propagated bounds of its inputs.  ``gmax``: the per-row top_db maxima
+    when ``E32`` holds only a window of the rows' frames (default: the maxima of ``E32``'s groups)."""
     E = E32.astype(np.float64)
     R, nfil, nF = E.shape
     if case.log == "db":
         x_db = 10.0 * np.log10(np.maximum(E, 1e-10))
         mag = np.abs(x_db)
         if case.top_db is not None:
-            gmax = np.array([E[(r // group) * group:(r // group + 1) * group].max() for r in range(R)])
+            if gmax is None:
+                gmax = np.array([E[(r // group) * group:(r // group + 1) * group].max() for r in range(R)])
+            gmax = np.asarray(gmax, np.float64)
             floor = 10.0 * np.log10(np.maximum(gmax, 1e-10)) - case.top_db
             y = np.maximum(x_db, floor[:, None, None])
             mag = np.maximum(mag, np.abs(floor)[:, None, None])
