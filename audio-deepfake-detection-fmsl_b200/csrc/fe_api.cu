@@ -12,8 +12,6 @@
 
 namespace {
 
-thread_local int64_t g_launches = 0;
-
 // Energies of one chunk of rows (the workspace between the energies kernel and the tail).  Round 1 kept a chunk inside
 // the 126 MB L2 (48 MB); measured on B200 the launch ramps and tails of three small launches cost more than the extra
 // 64 KB per utterance of DRAM traffic when the energies spill (the path runs at a quarter of the HBM roofline):
@@ -97,7 +95,7 @@ int32_t common_checks(const b200fe_params* p, const void* wave, int64_t R, int64
 
 }  // namespace
 
-extern "C" int64_t b200fe_last_launch_count(void) { return g_launches; }
+extern "C" int64_t b200fe_last_launch_count(void) { return fe_launch_count; }
 
 extern "C" int32_t b200fe_has_tcgen05(void) { return fe_gemm_compiled(); }
 
@@ -116,15 +114,15 @@ extern "C" int32_t b200fe_resolve_variant(const b200fe_params* p) {
   return (ok && fe_gemm_preferred(p)) ? B200FE_VARIANT_DFT_GEMM : B200FE_VARIANT_FFT;
 }
 
-// The streaming tcgen05 kernel fetches dense rows with TMA boxes: ragged clips and pre-emphasised input are
-// first written as dense rows (one chunk at a time) into the workspace.
-static bool needs_dense_rows(const b200fe_params* p, bool ragged) {
-  return p->variant == B200FE_VARIANT_DFT_GEMM && (ragged || p->preemph != 0.0f);
+// Whether a forward call first writes each chunk's rows as dense float32 rows into the workspace: 16-bit PCM (pcm16),
+// which both kernel families read only that way, and ragged clips or pre-emphasised input on the tensor cores, whose
+// streaming kernel fetches dense rows with TMA boxes.
+static bool stages_rows(const b200fe_params* p, bool ragged, bool pcm16) {
+  return pcm16 || (p->variant == B200FE_VARIANT_DFT_GEMM && (ragged || p->preemph != 0.0f));
 }
 
-// pcm16: 16-bit PCM input, which both kernel families read only as staged dense float32 rows
 static int64_t dense_rows_bytes(const b200fe_params* p, bool ragged, bool pcm16, int64_t chunk, int64_t T) {
-  return (pcm16 || needs_dense_rows(p, ragged)) ? ((chunk * T * 4 + 255) & ~(int64_t)255) : 0;
+  return stages_rows(p, ragged, pcm16) ? ((chunk * T * 4 + 255) & ~(int64_t)255) : 0;
 }
 
 static int64_t features_workspace_bytes(const b200fe_params* p, int64_t R, int64_t T, bool ragged, bool pcm16) {
@@ -151,7 +149,7 @@ extern "C" int64_t b200fe_workspace_bytes(const b200fe_params* p, int64_t R, int
 
 extern "C" int32_t b200fe_spectrogram_forward(const float* wave, int64_t R, int64_t T, const b200fe_params* p,
                                               const void* tables, float* out, void* stream) {
-  g_launches = 0;
+  fe_launch_count = 0;
   int32_t st = common_checks(p, wave, R, T, tables, out);
   if (st != B200FE_OK) return st;
   const int n_freq = p->n_fft / 2 + 1;
@@ -172,17 +170,8 @@ extern "C" int32_t b200fe_spectrogram_forward(const float* wave, int64_t R, int6
   a.radix2_first = (__builtin_ctz(p->n_fft / 2) & 1);
   a.top_db_group = 1;
   a.preemph = p->preemph;
-  // keep each launch's grid below 2^31 CTAs
-  const int64_t max_rows = 0x7fffffffLL / a.tiles_per_row;
-  for (int64_t r0 = 0; r0 < R; r0 += max_rows) {
-    const int64_t nr = R - r0 < max_rows ? R - r0 : max_rows;
-    a.row_base = r0;
-    a.out = out + (size_t)r0 * n_freq * a.n_frames;
-    cudaError_t e = fe_launch_fft(a, 0, nr, (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(e, "spectrogram kernel launch");
-    ++g_launches;
-  }
-  return B200FE_OK;
+  cudaError_t e = fe_launch_fft(a, 0, R, (cudaStream_t)stream);
+  return e == cudaSuccess ? B200FE_OK : cuda_fail(e, "spectrogram kernel launch");
 }
 
 // wave: float32 samples, or 16-bit PCM (pcm16: ragged only; every row is staged as dense float32 rows, x / 32768)
@@ -190,7 +179,6 @@ static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T,
                             const int32_t* lengths, const b200fe_params* p, const void* tables,
                             float* out, void* workspace, size_t workspace_bytes, void* stream_,
                             bool energies_only) {
-  g_launches = 0;
   const float* wave = (const float*)wave_;
   int32_t st = common_checks(p, wave_, R, T, tables, out, pcm16 ? 2 : 4);
   if (st != B200FE_OK) return st;
@@ -200,6 +188,7 @@ static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T,
     return B200FE_ERR_BAD_ARG;
   }
   if (p->n_filter < 1) { fe_set_error("n_filter must be >= 1 for the feature path"); return B200FE_ERR_BAD_ARG; }
+  const bool staged = stages_rows(p, offsets != nullptr, pcm16);
   const int64_t need = features_workspace_bytes(p, R, T, offsets != nullptr, pcm16);
   if (need < 0) return (int32_t)need;
   if (!workspace || workspace_bytes < (size_t)need) {
@@ -219,7 +208,7 @@ static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T,
       fe_set_error("variant dft_gemm needs T %% 4 == 0 and T > n_fft/2 (T=%lld, n_fft=%d)", (long long)T, p->n_fft);
       return B200FE_ERR_UNSUPPORTED;
     }
-    if (!pcm16 && !needs_dense_rows(p, offsets != nullptr) && ((uintptr_t)wave & 15) != 0) {
+    if (!staged && ((uintptr_t)wave & 15) != 0) {
       fe_set_error("variant dft_gemm needs a 16-byte aligned waveform (TMA)");
       return B200FE_ERR_UNSUPPORTED;
     }
@@ -233,7 +222,6 @@ static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T,
   unsigned int* gmax = needs_group_max(p) ? (unsigned int*)workspace : nullptr;
   float* energies = (float*)((char*)workspace + group_max_bytes(p, R));
   float* dense = (float*)((char*)energies + ((fe_align16(chunk * p->n_filter * (int64_t)n_frames * 4) + 255) & ~(int64_t)255));
-  const bool staged = pcm16 || (variant == B200FE_VARIANT_DFT_GEMM && needs_dense_rows(p, offsets != nullptr));
   void* gemm_ws = (char*)dense + dense_rows_bytes(p, offsets != nullptr, pcm16, chunk, T);
   const size_t row_energy_floats = (size_t)p->n_filter * n_frames;
 
@@ -293,82 +281,55 @@ static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T,
   for (int64_t r0 = 0; r0 < R; r0 += chunk) {
     const int64_t nr = R - r0 < chunk ? R - r0 : chunk;
     cudaError_t e;
-    if (energies_only) fa.out = out + (size_t)r0 * row_energy_floats;
-    if (pcm16) {
-      // every row staged (pre-emphasis included), then read as dense rows of this chunk by either kernel family
-      e = fe_launch_dense_rows((const int16_t*)wave_, offsets, lengths, r0, nr, T, p->preemph, dense, stream);
+    fe_fft_args fs = fa;
+    if (energies_only) fs.out = out + (size_t)r0 * row_energy_floats;
+    if (staged) {
+      // Float32 ragged clips that pad() only truncates (len >= T) and that start 16-byte aligned are read by the
+      // streaming kernel where they lie (the tensor maps then count 16-byte units above the lower of the two buffers);
+      // only the others -- short clips (repeat-pad), unaligned ones, and everything when pre-emphasis is on -- are staged.
+      int64_t flat_rel = -1, dense_rel = 0;
+      const float* base = dense;
+      if (!pcm16 && offsets && variant == B200FE_VARIANT_DFT_GEMM && p->preemph == 0.0f &&
+          ((uintptr_t)wave & 15) == 0 && !getenv("B200FE_STAGE_ALL")) {
+        const uintptr_t lo = (uintptr_t)wave < (uintptr_t)dense ? (uintptr_t)wave : (uintptr_t)dense;
+        const int64_t fr = (int64_t)(((uintptr_t)wave - lo) / 4), dr = (int64_t)(((uintptr_t)dense - lo) / 4);
+        if (((dr + nr * T) >> 2) < kFeInPlaceReach) {
+          base = (const float*)lo;
+          flat_rel = fr;
+          dense_rel = dr;
+        }
+      }
+      e = pcm16 ? fe_launch_dense_rows((const int16_t*)wave_, offsets, lengths, r0, nr, T, p->preemph, dense, stream)
+                : fe_launch_dense_rows(wave, offsets, lengths, r0, nr, T, p->preemph, dense, stream, flat_rel);
       if (e != cudaSuccess) return cuda_fail(e, "dense-rows kernel launch");
-      g_launches += (nr + 65534) / 65535;
-      fe_fft_args fs = fa;
-      fs.wave = nullptr;
       fs.wave_chunk = dense;
-      fs.offsets = nullptr;
-      fs.lengths = nullptr;
       fs.preemph = 0.0f;
-      if (variant == B200FE_VARIANT_DFT_GEMM) {
-        int launches = 0;
-        e = fe_stream_launch(p, fs, r0, nr, gemm_ws, stream, &launches);
-        if (e != cudaSuccess) return cuda_fail(e, "dft-gemm kernel launch");
-        g_launches += launches;
+      if (flat_rel >= 0) {
+        fs.wave = base;
+        fs.in_place = 1;
+        fs.flat_rel = flat_rel;
+        fs.dense_rel = dense_rel;
       } else {
-        fs.row_base = r0;
-        e = fe_launch_fft(fs, 1, nr, stream);
-        if (e != cudaSuccess) return cuda_fail(e, "fft kernel launch");
-        ++g_launches;
+        fs.offsets = nullptr;
+        fs.lengths = nullptr;
       }
-    } else if (variant == B200FE_VARIANT_DFT_GEMM) {
-      int launches = 0;
-      if (staged) {
-        // Ragged clips that pad() only truncates (len >= T) and that start 16-byte aligned are read where they lie
-        // (the tensor maps then count 16-byte units above the lower of the two buffers); only the others -- short
-        // clips (repeat-pad), unaligned ones, and everything when pre-emphasis is on -- are staged as dense rows.
-        int64_t flat_rel = -1, dense_rel = 0;
-        const float* base = dense;
-        if (offsets && lengths && p->preemph == 0.0f && ((uintptr_t)wave & 15) == 0 && !getenv("B200FE_STAGE_ALL")) {
-          const uintptr_t lo = (uintptr_t)wave < (uintptr_t)dense ? (uintptr_t)wave : (uintptr_t)dense;
-          const int64_t fr = (int64_t)(((uintptr_t)wave - lo) / 4), dr = (int64_t)(((uintptr_t)dense - lo) / 4);
-          if (((dr + nr * T) >> 2) < kFeInPlaceReach) {
-            base = (const float*)lo;
-            flat_rel = fr;
-            dense_rel = dr;
-          }
-        }
-        e = fe_launch_dense_rows(wave, offsets, lengths, r0, nr, T, p->preemph, dense, stream, flat_rel);
-        if (e != cudaSuccess) return cuda_fail(e, "dense-rows kernel launch");
-        g_launches += (nr + 65534) / 65535;
-        fe_fft_args fs = fa;
-        fs.wave_chunk = dense;
-        if (flat_rel >= 0) {
-          fs.wave = base;
-          fs.in_place = 1;
-          fs.flat_rel = flat_rel;
-          fs.dense_rel = dense_rel;
-        } else {
-          fs.offsets = nullptr;
-          fs.lengths = nullptr;
-        }
-        e = fe_stream_launch(p, fs, r0, nr, gemm_ws, stream, &launches);
-      } else {
-        e = fe_stream_launch(p, fa, r0, nr, gemm_ws, stream, &launches);
-      }
+    }
+    if (variant == B200FE_VARIANT_DFT_GEMM) {
+      e = fe_stream_launch(p, fs, r0, nr, gemm_ws, stream);
       if (e != cudaSuccess) return cuda_fail(e, "dft-gemm kernel launch");
-      g_launches += launches;
     } else {
-      fa.row_base = r0;
-      e = fe_launch_fft(fa, 1, nr, stream);
+      fs.row_base = r0;
+      e = fe_launch_fft(fs, 1, nr, stream);
       if (e != cudaSuccess) return cuda_fail(e, "fft kernel launch");
-      ++g_launches;
     }
     if (energies_only) continue;
     ta.row_base = r0;
     e = fe_launch_tail(ta, nr, stream);
     if (e != cudaSuccess) return cuda_fail(e, "tail kernel launch");
-    g_launches += (nr + 65534) / 65535;
   }
   if (p->cmvn && !energies_only) {
     cudaError_t e = fe_launch_cmvn(out, R * n_out, n_frames, stream);
     if (e != cudaSuccess) return cuda_fail(e, "cmvn kernel launch");
-    ++g_launches;
   }
   return B200FE_OK;
 }
@@ -376,38 +337,43 @@ static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T,
 extern "C" int32_t b200fe_features_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
                                            const int32_t* lengths, const b200fe_params* p, const void* tables,
                                            float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  fe_launch_count = 0;
   return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
 }
 
 extern "C" int32_t b200fe_features_forward_ragged_i16(const int16_t* pcm, int64_t R, int64_t T, const int64_t* offsets,
                                                       const int32_t* lengths, const b200fe_params* p, const void* tables,
                                                       float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  fe_launch_count = 0;
   return run_features(pcm, true, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
 }
 
 extern "C" int32_t b200fe_fbank_energies_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
                                                  const int32_t* lengths, const b200fe_params* p, const void* tables,
                                                  float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  fe_launch_count = 0;
   return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, true);
 }
 
 extern "C" int32_t b200fe_lfcc_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
                                        const int32_t* lengths, const b200fe_params* p, const void* tables,
                                        float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  fe_launch_count = 0;
   if (p && p->n_coef < 1) { fe_set_error("b200fe_lfcc_forward needs n_coef >= 1"); return B200FE_ERR_BAD_ARG; }
-  return b200fe_features_forward(wave, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream);
+  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
 }
 
 extern "C" int32_t b200fe_mel_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
                                       const int32_t* lengths, const b200fe_params* p, const void* tables,
                                       float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  fe_launch_count = 0;
   if (p && p->n_coef != 0) { fe_set_error("b200fe_mel_forward needs n_coef == 0"); return B200FE_ERR_BAD_ARG; }
-  return b200fe_features_forward(wave, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream);
+  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
 }
 
 extern "C" int32_t b200fe_compute_deltas(const float* in, int64_t rows, int64_t T, int32_t win, float* out,
                                          void* stream) {
-  g_launches = 0;
+  fe_launch_count = 0;
   if (!in || !out) { fe_set_error("in / out is NULL"); return B200FE_ERR_BAD_ARG; }
   if (rows < 1 || T < 1) { fe_set_error("rows=%lld T=%lld must be >= 1", (long long)rows, (long long)T); return B200FE_ERR_BAD_ARG; }
   if (win < 3) { fe_set_error("win_length=%d must be >= 3", win); return B200FE_ERR_BAD_ARG; }
@@ -416,7 +382,6 @@ extern "C" int32_t b200fe_compute_deltas(const float* in, int64_t rows, int64_t 
   if (st != B200FE_OK) return st;
   cudaError_t e = fe_launch_deltas(in, out, rows, T, win, (cudaStream_t)stream);
   if (e != cudaSuccess) return cuda_fail(e, "deltas kernel launch");
-  g_launches = (rows + 65534) / 65535;
   return B200FE_OK;
 }
 
@@ -440,10 +405,11 @@ struct host_slot_layout {
   int64_t in_bytes, idx_bytes, wave_bytes, out_bytes, ws_bytes, slot_bytes;
 };
 
-// params of the dense forward call of a ragged chunk: pre-emphasis is applied while the rows are staged
-b200fe_params staged_params(const b200fe_params* p) {
+// params of the dense forward call of a chunk: ragged and 16-bit PCM chunks are staged as float32 rows first, and
+// pre-emphasis is applied while they are staged
+b200fe_params chunk_params(const b200fe_params* p, int32_t sample_bytes, bool ragged) {
   b200fe_params q = *p;
-  q.preemph = 0.0f;
+  if (ragged || sample_bytes == 2) q.preemph = 0.0f;
   return q;
 }
 
@@ -452,7 +418,7 @@ int32_t host_layout(const b200fe_params* p, int64_t chunk_rows, int64_t T, int32
   const int64_t nf = b200fe_n_frames(p, T);
   if (nf < 0) return (int32_t)nf;
   const int64_t n_out = b200fe_n_out_channels(p);
-  const b200fe_params q = ragged ? staged_params(p) : *p;
+  const b200fe_params q = chunk_params(p, sample_bytes, ragged);
   const int64_t ws = b200fe_workspace_bytes(&q, chunk_rows, T);
   if (ws < 0) return (int32_t)ws;
   if (ragged) {
@@ -521,14 +487,14 @@ int64_t ragged_chunk(const host_input& in, int64_t r0, int64_t max_rows, int64_t
 }
 
 // One loop for dense rows and ragged clips; a chunk goes to stream c % n_streams and its slot:
-//   dense:  H2D rows -> (16-bit PCM: x / 32768) -> dense forward -> D2H features
-//   ragged: H2D copy span, H2D clip table slice -> stage dense rows (pad(), x / 32768, pre-emphasis) -> dense forward
+//   dense float32: H2D rows -> dense forward -> D2H features
+//   dense 16-bit PCM: H2D rows -> stage float32 rows (x / 32768, pre-emphasis) -> dense forward without pre-emphasis
+//                     -> D2H features
+//   ragged: H2D copy span, H2D clip table slice -> stage float32 rows (pad(), x / 32768, pre-emphasis) -> dense forward
 //           without pre-emphasis -> D2H features
 int32_t forward_host(const host_input& in, int64_t R, int64_t T, const b200fe_params* p, const void* tables,
                      float* out_host, void* staging, size_t staging_bytes, int64_t chunk_rows, void* const* streams,
                      int32_t n_streams) {
-  int64_t launches = 0;
-  g_launches = 0;
   const bool ragged = in.offsets != nullptr;
   if (!in.data || !out_host || !staging || !streams || !p) { fe_set_error("NULL argument"); return B200FE_ERR_BAD_ARG; }
   if (R < 1) { fe_set_error("R=%lld must be >= 1", (long long)R); return B200FE_ERR_BAD_ARG; }
@@ -549,7 +515,7 @@ int32_t forward_host(const host_input& in, int64_t R, int64_t T, const b200fe_pa
   }
   host_slot_layout L;
   host_layout(p, chunk_rows, T, in.sample_bytes, ragged, &L);
-  const b200fe_params q = ragged ? staged_params(p) : *p;
+  const b200fe_params q = chunk_params(p, in.sample_bytes, ragged);
   const int64_t nf = b200fe_n_frames(p, T);
   const int64_t n_out = b200fe_n_out_channels(p);
   const size_t in_elt = (size_t)in.sample_bytes;
@@ -568,20 +534,17 @@ int32_t forward_host(const host_input& in, int64_t R, int64_t T, const b200fe_pa
     float* d_wave = (float*)(d_idx + L.idx_bytes);
     float* d_out = (float*)((char*)d_wave + L.wave_bytes);
     void* d_ws = (char*)d_out + L.out_bytes;
+    int64_t* d_off = nullptr;
+    int32_t* d_len = nullptr;
     cudaError_t e;
     if (!ragged) {
       // one copy per chunk and direction
       e = cudaMemcpyAsync(pcm16 ? d_in : (void*)d_wave, (const char*)in.data + (size_t)r0 * T * in_elt,
                           (size_t)nr * T * in_elt, cudaMemcpyHostToDevice, st);
       if (e != cudaSuccess) return cuda_fail(e, "H2D copy");
-      if (pcm16) {
-        e = fe_launch_i16_rows((const int16_t*)d_in, d_wave, nr * T, st);
-        if (e != cudaSuccess) return cuda_fail(e, "pcm16 conversion kernel launch");
-        ++launches;
-      }
     } else {
-      int64_t* d_off = (int64_t*)d_idx;
-      int32_t* d_len = (int32_t*)(d_idx + ((chunk_rows * 8 + 255) & ~(int64_t)255));
+      d_off = (int64_t*)d_idx;
+      d_len = (int32_t*)(d_idx + ((chunk_rows * 8 + 255) & ~(int64_t)255));
       e = cudaMemcpyAsync(d_in, (const char*)in.data + (size_t)lo * in_elt, (size_t)(hi - lo) * in_elt,
                           cudaMemcpyHostToDevice, st);
       if (e != cudaSuccess) return cuda_fail(e, "H2D copy");
@@ -589,14 +552,15 @@ int32_t forward_host(const host_input& in, int64_t R, int64_t T, const b200fe_pa
       if (e != cudaSuccess) return cuda_fail(e, "H2D copy (offsets)");
       e = cudaMemcpyAsync(d_len, in.lengths + r0, (size_t)nr * 4, cudaMemcpyHostToDevice, st);
       if (e != cudaSuccess) return cuda_fail(e, "H2D copy (lengths)");
+    }
+    if (ragged || pcm16) {
       e = pcm16 ? fe_launch_dense_rows((const int16_t*)d_in, d_off, d_len, 0, nr, T, p->preemph, d_wave, st, lo)
                 : fe_launch_dense_rows((const float*)d_in, d_off, d_len, 0, nr, T, p->preemph, d_wave, st, -1, lo);
       if (e != cudaSuccess) return cuda_fail(e, "dense-rows kernel launch");
-      launches += (nr + 65534) / 65535;
     }
-    int32_t rc = b200fe_features_forward(d_wave, nr, T, nullptr, nullptr, &q, tables, d_out, d_ws, (size_t)L.ws_bytes, st);
+    int32_t rc = run_features(d_wave, false, nr, T, nullptr, nullptr, &q, tables, d_out, d_ws, (size_t)L.ws_bytes, st,
+                              false);
     if (rc != B200FE_OK) return rc;
-    launches += g_launches;
     e = cudaMemcpyAsync(out_host + (size_t)r0 * n_out * nf, d_out, (size_t)nr * n_out * nf * 4, cudaMemcpyDeviceToHost, st);
     if (e != cudaSuccess) return cuda_fail(e, "D2H copy");
     r0 += nr;
@@ -605,7 +569,6 @@ int32_t forward_host(const host_input& in, int64_t R, int64_t T, const b200fe_pa
     cudaError_t e = cudaStreamSynchronize((cudaStream_t)streams[s]);
     if (e != cudaSuccess) return cuda_fail(e, "cudaStreamSynchronize");
   }
-  g_launches = launches;
   return B200FE_OK;
 }
 
@@ -629,6 +592,7 @@ extern "C" int32_t b200fe_features_forward_host(const float* wave_host, int64_t 
                                                 const void* tables, float* out_host, void* staging,
                                                 size_t staging_bytes, int64_t chunk_rows, void* const* streams,
                                                 int32_t n_streams) {
+  fe_launch_count = 0;
   return forward_host(dense_input(wave_host, 4), R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams,
                       n_streams);
 }
@@ -637,6 +601,7 @@ extern "C" int32_t b200fe_features_forward_host_i16(const int16_t* pcm_host, int
                                                     const void* tables, float* out_host, void* staging,
                                                     size_t staging_bytes, int64_t chunk_rows, void* const* streams,
                                                     int32_t n_streams) {
+  fe_launch_count = 0;
   return forward_host(dense_input(pcm_host, 2), R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams,
                       n_streams);
 }
@@ -646,7 +611,7 @@ extern "C" int32_t b200fe_features_forward_host_ragged(const void* clips_host, i
                                                        int64_t R, int64_t T, const b200fe_params* p, const void* tables,
                                                        float* out_host, void* staging, size_t staging_bytes,
                                                        int64_t chunk_rows, void* const* streams, int32_t n_streams) {
-  g_launches = 0;
+  fe_launch_count = 0;
   if (!offsets_host || !lengths_host) { fe_set_error("offsets / lengths is NULL"); return B200FE_ERR_BAD_ARG; }
   if (n_samples < 1) { fe_set_error("n_samples=%lld must be >= 1", (long long)n_samples); return B200FE_ERR_BAD_ARG; }
   const host_input in{clips_host, sample_bytes, offsets_host, lengths_host, n_samples};

@@ -13,7 +13,7 @@ int64_t fe_gemm_workspace_bytes(const b200fe_params* p, int64_t chunk_rows, int6
 // T > n_fft/2, at least two frames).  Any row count is taken: fe_stream_launch splits the rows into launches.
 bool fe_stream_supported(const b200fe_params* p, int64_t T);
 // Filterbank energies (+ group maxima) of rows [row_base, row_base+rows) into fa.out, like fe_launch_fft(mode 1), in
-// as many launches (*launches) as the kernel's 32-bit frame and element indices need.
+// as many launches as the kernel's 32-bit frame and element indices need.
 cudaError_t fe_stream_launch(const b200fe_params* p, const fe_fft_args& fa, int64_t row_base, int64_t rows,
-                             void* gemm_ws, cudaStream_t stream, int* launches);
+                             void* gemm_ws, cudaStream_t stream);
 #endif

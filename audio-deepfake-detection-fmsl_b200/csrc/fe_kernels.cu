@@ -934,9 +934,9 @@ __global__ void fe_deltas_kernel(const float* __restrict__ in, float* __restrict
 // and / or pre-emphasis -> dense rows [rows][T] the streaming tcgen05 kernel can fetch with TMA boxes.
 // One thread = four consecutive samples of one row, one 16-byte store (VEC4: T % 4 == 0; otherwise four scalar stores,
 // for the FFT variant, which reads dense rows of any T).  Samples are float32 or 16-bit PCM converted as x / 32768
-// (the expression of fe_i16_rows_kernel), read one at a time: an int16 clip may start on any 2-byte boundary.
-// Row r's clip starts offsets[r] - base samples into `wave`, which then holds only the span of the flat clip buffer
-// from sample `base` on.
+// (exact in fp32: what a FLAC / WAV decoder's float conversion yields), read one at a time: an int16 clip may start on
+// any 2-byte boundary.  Row r's clip starts offsets[r] - base samples into `wave`, which then holds only the span of
+// the flat clip buffer from sample `base` on; without offsets, `wave` holds dense rows [rows][T].
 // ------------------------------------------------------------------------------------------------
 FE_HD float fe_sample_f32(float x) { return x; }
 FE_HD float fe_sample_f32(int16_t x) { return (1.0f / 32768.0f) * (float)x; }
@@ -983,21 +983,6 @@ __global__ void __launch_bounds__(256) fe_dense_rows_kernel(const S* __restrict_
 }
 
 // ------------------------------------------------------------------------------------------------
-// fe_i16_rows_kernel : 16-bit PCM rows -> float32 rows, x / 32768 (exact in fp32: what a FLAC / WAV decoder's
-// float conversion yields, maze5.py:297-351 via librosa / soundfile).  One thread = four samples.
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) fe_i16_rows_kernel(const int16_t* __restrict__ src, float* __restrict__ dst,
-                                                         int64_t n4, int64_t n) {
-  const float k = 1.0f / 32768.0f;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
-    const short4 v = reinterpret_cast<const short4*>(src)[i];
-    reinterpret_cast<float4*>(dst)[i] = make_float4(k * (float)v.x, k * (float)v.y, k * (float)v.z, k * (float)v.w);
-  }
-  if (blockIdx.x == 0)
-    for (int64_t i = 4 * n4 + threadIdx.x; i < n; i += blockDim.x) dst[i] = k * (float)src[i];
-}
-
-// ------------------------------------------------------------------------------------------------
 // fe_tail_pointwise_kernel : the tail when there is no DCT and no deltas (mel features): out = log/dB(energies)
 // element by element with the arithmetic of fe_tail_load; a row's [n_filter][n_frames] block is contiguous on
 // both sides.  grid (blocks per row, rows), 4 elements per thread, coalesced.
@@ -1034,6 +1019,8 @@ cudaError_t set_smem(const void* fn, size_t bytes) {
 }
 
 }  // namespace
+
+thread_local int64_t fe_launch_count = 0;
 
 cudaError_t fe_ensure_smem(const void* fn, size_t bytes) {
   // The opt-in is process-wide per (function, device), and it costs a microsecond or two per call, which a small-batch
@@ -1125,8 +1112,6 @@ cudaError_t fe_launch_fft(const fe_fft_args& a_in, int mode, int64_t rows, cudaS
   a.fft_warps = fe_fft_warps_for(a.n_fft);
   const int n_ch = mode == 0 ? a.n_fft / 2 + 1 : a.n_filter;
   const size_t smem = fe_fft_smem_bytes(a.n_fft, a.hop, a.ft, n_ch, mode);
-  const int64_t grid = rows * a.tiles_per_row;
-  if (grid <= 0 || grid > 0x7fffffffLL) return cudaErrorInvalidConfiguration;
   const int E = fe_fft_fast_e(a.n_fft, a.hop);
   void (*kern)(fe_fft_args);
   switch (E * 2 + (mode != 0)) {
@@ -1141,18 +1126,24 @@ cudaError_t fe_launch_fft(const fe_fft_args& a_in, int mode, int64_t rows, cudaS
   }
   cudaError_t e = set_smem((const void*)kern, smem);
   if (e != cudaSuccess) return e;
-  int64_t launch_grid = grid;
+  int64_t resident = 0x7fffffffLL;
   if (E > 0) {   // persistent CTAs: as many as are resident at once
     const int sms = fe_device_sms(fe_current_device());
     int per_sm = 1;
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kFftThreads, smem);
     if (e != cudaSuccess) return e;
-    a.n_blocks = grid;
-    const int64_t resident = (int64_t)sms * (per_sm > 0 ? per_sm : 1);
-    if (launch_grid > resident) launch_grid = resident;
+    resident = (int64_t)sms * (per_sm > 0 ? per_sm : 1);
   }
-  kern<<<(unsigned)launch_grid, kFftThreads, smem, stream>>>(a);
-  return cudaGetLastError();
+  // one CTA per (row, tile): keep each launch's grid below 2^31 CTAs; `out` and `wave_chunk` hold the launch's rows
+  return fe_launch_rows(rows, 0x7fffffffLL / a.tiles_per_row, [&](int64_t r0, int64_t nr) {
+    fe_fft_args b = a;
+    b.row_base = a.row_base + r0;
+    b.out = a.out + (size_t)r0 * n_ch * a.n_frames;
+    if (a.wave_chunk) b.wave_chunk = a.wave_chunk + r0 * a.T;
+    b.n_blocks = nr * a.tiles_per_row;
+    kern<<<(unsigned)(b.n_blocks < resident ? b.n_blocks : resident), kFftThreads, smem, stream>>>(b);
+    return cudaSuccess;
+  });
 }
 
 size_t fe_tail_smem_bytes(const fe_tail_args& a) {
@@ -1163,6 +1154,14 @@ size_t fe_tail_smem_bytes(const fe_tail_args& a) {
   if (a.deltas > 0) fl += (size_t)nc * w;
   fl += (size_t)a.n_filter * a.n_coef;
   return fl * 4;
+}
+
+// The tail arguments of a launch over rows [r0, ...) of a's rows (energies hold a's rows from a.row_base on).
+static fe_tail_args tail_rows_from(const fe_tail_args& a, int64_t r0) {
+  fe_tail_args b = a;
+  b.row_base = a.row_base + r0;
+  b.energies = a.energies + (size_t)r0 * a.n_filter * a.n_frames;
+  return b;
 }
 
 template <int N, bool EXACT>
@@ -1209,18 +1208,12 @@ static bool launch_tail_quad(const fe_tail_args& a_in, int64_t rows, cudaStream_
   }
   *err = set_smem((const void*)kern, smem);
   if (*err != cudaSuccess) return true;
-  // one CTA per (row, tile), a 1-D grid (no 65535-row limit)
-  const int64_t max_rows = (int64_t)0x3fffffff / tiles;   // tile indices (and index + grid) are 32-bit in the kernel
-  for (int64_t r0 = 0; r0 < rows; r0 += max_rows) {
-    fe_tail_args b = a;
-    const int64_t nr = rows - r0 < max_rows ? rows - r0 : max_rows;
-    b.row_base = a.row_base + r0;
-    b.energies = a.energies + (size_t)r0 * a.n_filter * a.n_frames;
-    const int64_t n_tiles = nr * tiles;
-    kern<<<(unsigned)n_tiles, threads, smem, stream>>>(b, tiles, (int)n_tiles);
-    *err = cudaGetLastError();
-    if (*err != cudaSuccess) return true;
-  }
+  // one CTA per (row, tile), a 1-D grid (no 65535-row limit); tile indices (and index + grid) are 32-bit in the kernel
+  *err = fe_launch_rows(rows, (int64_t)0x3fffffff / tiles, [&](int64_t r0, int64_t nr) {
+    const int n_tiles = (int)(nr * tiles);
+    kern<<<(unsigned)n_tiles, threads, smem, stream>>>(tail_rows_from(a, r0), tiles, n_tiles);
+    return cudaSuccess;
+  });
   return true;
 }
 
@@ -1247,33 +1240,20 @@ static cudaError_t launch_tail_fast(const fe_tail_args& a_in, int64_t rows, cuda
                             : (n == 2 ? pick_tail_fast<2, false>(kq) : pick_tail_fast<0, false>(kq));
   cudaError_t e = set_smem((const void*)kern, smem);
   if (e != cudaSuccess) return e;
-  for (int64_t r0 = 0; r0 < rows; r0 += 65535) {
-    fe_tail_args b = a;
-    const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
-    b.row_base = a.row_base + r0;
-    b.energies = a.energies + (size_t)r0 * a.n_filter * a.n_frames;
-    dim3 grid((unsigned)tiles, (unsigned)nr);
-    kern<<<grid, threads, smem, stream>>>(b);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-  }
-  return cudaSuccess;
+  return fe_launch_rows(rows, 65535, [&](int64_t r0, int64_t nr) {
+    kern<<<dim3((unsigned)tiles, (unsigned)nr), threads, smem, stream>>>(tail_rows_from(a, r0));
+    return cudaSuccess;
+  });
 }
 
 cudaError_t fe_launch_tail(const fe_tail_args& a, int64_t rows, cudaStream_t stream) {
   if (a.n_coef == 0 && a.deltas == 0 && a.force_generic != 1) {
     const int64_t per_row = (int64_t)a.n_filter * a.n_frames;
-    for (int64_t r0 = 0; r0 < rows; r0 += 65535) {
-      fe_tail_args b = a;
-      const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
-      b.row_base = a.row_base + r0;
-      b.energies = a.energies + (size_t)r0 * per_row;
-      dim3 grid((unsigned)((per_row + 1023) / 1024), (unsigned)nr);
-      fe_tail_pointwise_kernel<<<grid, 256, 0, stream>>>(b);
-      cudaError_t e = cudaGetLastError();
-      if (e != cudaSuccess) return e;
-    }
-    return cudaSuccess;
+    return fe_launch_rows(rows, 65535, [&](int64_t r0, int64_t nr) {
+      fe_tail_pointwise_kernel<<<dim3((unsigned)((per_row + 1023) / 1024), (unsigned)nr), 256, 0, stream>>>(
+          tail_rows_from(a, r0));
+      return cudaSuccess;
+    });
   }
   if (a.n_filter <= kFastMax && a.n_coef <= kFastMax && a.force_generic != 1) return launch_tail_fast(a, rows, stream);
   const size_t smem = fe_tail_smem_bytes(a);
@@ -1281,38 +1261,28 @@ cudaError_t fe_launch_tail(const fe_tail_args& a, int64_t rows, cudaStream_t str
   if (e != cudaSuccess) return e;
   const int tiles = (a.n_frames + a.tt - 1) / a.tt;
   // grid.y is limited to 65535 rows per launch
-  for (int64_t r0 = 0; r0 < rows; r0 += 65535) {
-    fe_tail_args b = a;
-    const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
-    b.row_base = a.row_base + r0;
-    b.energies = a.energies + (size_t)r0 * a.n_filter * a.n_frames;
-    dim3 grid((unsigned)tiles, (unsigned)nr);
-    fe_tail_kernel<<<grid, kTailThreads, smem, stream>>>(b);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-  }
-  return cudaSuccess;
+  return fe_launch_rows(rows, 65535, [&](int64_t r0, int64_t nr) {
+    fe_tail_kernel<<<dim3((unsigned)tiles, (unsigned)nr), kTailThreads, smem, stream>>>(tail_rows_from(a, r0));
+    return cudaSuccess;
+  });
 }
 
 cudaError_t fe_launch_cmvn(float* out, int64_t n_series, int n_frames, cudaStream_t stream) {
   const int warps = 8;
   const int64_t grid = (n_series + warps - 1) / warps;
   fe_cmvn_kernel<<<(unsigned)grid, warps * 32, 0, stream>>>(out, n_series, n_frames, 1e-5f);
-  return cudaGetLastError();
+  return fe_launched();
 }
 
 cudaError_t fe_launch_deltas(const float* in, float* out, int64_t rows, int64_t T, int win,
                              cudaStream_t stream) {
   const int n = (win - 1) / 2;
   const float denom = (float)(n * (n + 1) * (2 * n + 1)) / 3.0f;
-  for (int64_t r0 = 0; r0 < rows; r0 += 65535) {
-    const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
-    dim3 grid((unsigned)((T + 255) / 256), (unsigned)nr);
-    fe_deltas_kernel<<<grid, 256, 0, stream>>>(in + r0 * T, out + r0 * T, nr, T, n, denom);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-  }
-  return cudaSuccess;
+  return fe_launch_rows(rows, 65535, [&](int64_t r0, int64_t nr) {
+    fe_deltas_kernel<<<dim3((unsigned)((T + 255) / 256), (unsigned)nr), 256, 0, stream>>>(in + r0 * T, out + r0 * T,
+                                                                                         nr, T, n, denom);
+    return cudaSuccess;
+  });
 }
 
 template <typename S>
@@ -1327,8 +1297,7 @@ static cudaError_t launch_dense_rows(const S* wave, const int64_t* offsets, cons
   const unsigned cap = flat_rel >= 0 ? 8 : 16;
   if (bx > cap) bx = cap;
   const bool vec4 = (T & 3) == 0;
-  for (int64_t r0 = 0; r0 < rows; r0 += 65535) {
-    const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
+  return fe_launch_rows(rows, 65535, [&](int64_t r0, int64_t nr) {
     dim3 grid(bx, (unsigned)nr);
     if (vec4)
       fe_dense_rows_kernel<S, true><<<grid, 256, 0, stream>>>(wave, offsets, lengths, row_base + r0, (int)T, preemph,
@@ -1336,10 +1305,8 @@ static cudaError_t launch_dense_rows(const S* wave, const int64_t* offsets, cons
     else
       fe_dense_rows_kernel<S, false><<<grid, 256, 0, stream>>>(wave, offsets, lengths, row_base + r0, (int)T, preemph,
                                                                dst + r0 * T, flat_rel, base);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-  }
-  return cudaSuccess;
+    return cudaSuccess;
+  });
 }
 
 cudaError_t fe_launch_dense_rows(const float* wave, const int64_t* offsets, const int32_t* lengths,
@@ -1352,14 +1319,4 @@ cudaError_t fe_launch_dense_rows(const int16_t* wave, const int64_t* offsets, co
                                  int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
                                  cudaStream_t stream, int64_t base) {
   return launch_dense_rows(wave, offsets, lengths, row_base, rows, T, preemph, dst, stream, (int64_t)-1, base);
-}
-
-cudaError_t fe_launch_i16_rows(const int16_t* src, float* dst, int64_t n, cudaStream_t stream) {
-  // both pointers 8 / 16-byte aligned (staging slots are 256-byte aligned): vector body + scalar tail
-  const int64_t n4 = n / 4;
-  int64_t blocks = (n4 + 255) / 256;
-  if (blocks < 1) blocks = 1;
-  if (blocks > 148 * 16) blocks = 148 * 16;
-  fe_i16_rows_kernel<<<(unsigned)blocks, 256, 0, stream>>>(src, dst, n4, n);
-  return cudaGetLastError();
 }

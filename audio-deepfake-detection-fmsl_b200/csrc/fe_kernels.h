@@ -51,6 +51,28 @@ int fe_device_sms(int dev);         // multiprocessor count of `dev`
 // uncontended lock and no CUDA call.
 cudaError_t fe_ensure_smem(const void* fn, size_t bytes);
 
+// Kernels launched by this thread since the entry point that was called last reset it (b200fe_last_launch_count).
+extern thread_local int64_t fe_launch_count;
+
+// After a <<<>>>: the launch's error, counted in fe_launch_count when there is none.
+inline cudaError_t fe_launched(void) {
+  const cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) ++fe_launch_count;
+  return e;
+}
+
+// Rows [0, rows) in pieces of at most max_rows: launch(r0, nr) enqueues one kernel over rows [r0, r0 + nr), or returns
+// the error that kept it from doing so.  Stops at the first error.
+template <typename F>
+cudaError_t fe_launch_rows(int64_t rows, int64_t max_rows, F&& launch) {
+  for (int64_t r0 = 0; r0 < rows; r0 += max_rows) {
+    cudaError_t e = launch(r0, rows - r0 < max_rows ? rows - r0 : max_rows);
+    if (e == cudaSuccess) e = fe_launched();
+    if (e != cudaSuccess) return e;
+  }
+  return cudaSuccess;
+}
+
 // A ragged clip the streaming kernel can read where it lies: pad() only truncates it (len >= T), and its first sample
 // is 16-byte aligned relative to the tensor map's base and within the map's reach (32 steps of 32 GB above the base).
 // fe_dense_rows_kernel skips exactly these rows; fe_stream_kernel reads exactly these rows from the flat buffer.
@@ -77,6 +99,4 @@ cudaError_t fe_launch_dense_rows(const float* wave, const int64_t* offsets, cons
 cudaError_t fe_launch_dense_rows(const int16_t* wave, const int64_t* offsets, const int32_t* lengths,
                                  int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
                                  cudaStream_t stream, int64_t base = 0);
-// 16-bit PCM -> float32 (x / 32768), n samples; src 8-byte and dst 16-byte aligned.
-cudaError_t fe_launch_i16_rows(const int16_t* src, float* dst, int64_t n, cudaStream_t stream);
 #endif

@@ -750,7 +750,8 @@ bool fe_stream_supported(const b200fe_params* p, int64_t T) {
 namespace {
 
 // One launch of the streaming kernel over rows [row_base, row_base + rows) of the call, which keep the launch's frame
-// and element indices within 32 bits (fe_stream_launch).
+// and element indices within 32 bits (fe_stream_launch).  Returns the errors met before the launch; fe_launch_rows
+// checks the launch itself.
 cudaError_t stream_launch_one(const b200fe_params* p, const fe_fft_args& fa, int64_t row_base, int64_t rows,
                               void* gemm_ws, cudaStream_t stream) {
   stream_args a;
@@ -849,29 +850,23 @@ cudaError_t stream_launch_one(const b200fe_params* p, const fe_fft_args& fa, int
 #endif
   if (e != cudaSuccess) return e;
   fe_stream_kernel<<<grid, kThreads, smem, stream>>>(*maps_p, a);
-  return cudaGetLastError();
+  return cudaSuccess;
 }
 
 }  // namespace
 
 cudaError_t fe_stream_launch(const b200fe_params* p, const fe_fft_args& fa, int64_t row_base, int64_t rows,
-                             void* gemm_ws, cudaStream_t stream, int* launches) {
-  *launches = 0;
+                             void* gemm_ws, cudaStream_t stream) {
   // The kernel indexes a launch's frames (fe_tile_geometry: frames plus one hop block per row) and energy elements
   // (emit_store) in 32 bits: rows * n_frames < 2^30 and rows * n_filter * n_frames < 2^31 per launch.  One row always
   // fits (T < 2^30, hop >= 32, n_filter <= 32).
   const int64_t nF = fa.n_frames, per_row = (int64_t)p->n_filter * nF;
   const int64_t frame_rows = (((int64_t)1 << 30) - 1) / nF, energy_rows = (((int64_t)1 << 31) - 1) / per_row;
-  const int64_t max_rows = frame_rows < energy_rows ? frame_rows : energy_rows;
-  for (int64_t r0 = 0; r0 < rows; r0 += max_rows) {
-    const int64_t nr = rows - r0 < max_rows ? rows - r0 : max_rows;
+  return fe_launch_rows(rows, frame_rows < energy_rows ? frame_rows : energy_rows, [&](int64_t r0, int64_t nr) {
     fe_fft_args f = fa;
     f.out = fa.out + r0 * per_row;
     if (fa.wave_chunk) f.wave_chunk = fa.wave_chunk + r0 * fa.T;
     f.dense_rel = fa.dense_rel + r0 * fa.T;
-    cudaError_t e = stream_launch_one(p, f, row_base + r0, nr, gemm_ws, stream);
-    if (e != cudaSuccess) return e;
-    ++*launches;
-  }
-  return cudaSuccess;
+    return stream_launch_one(p, f, row_base + r0, nr, gemm_ws, stream);
+  });
 }

@@ -329,5 +329,4 @@ CASES = _energy_cases() + _stream_cases() + _quad_cases() + _fast_cases() + _gen
 ALLOWLIST = {
     "fe_eer_kernel": "test_gpu_fullsize::test_device_eer_equals_sklearn_digit_for_digit",
     "fe_cmvn_kernel": "test_gpu_parity::test_cmvn_extension",
-    "fe_i16_rows_kernel": "test_gpu_fullsize::test_pcm16_host_path_is_bit_identical_to_float_path",
 }
