@@ -5,6 +5,11 @@ CUDA behind a C-ABI (``include/b200fe.h``).  The modules keep torchaudio's const
 and ``(..., C, n_frames)`` output layout so they drop into the reference's feature slot
 (``model.sinc_conv``, Thesis/01_Models/01_Baseline_Models/maze5.py:241).
 
+Variable-length clips (``forward_ragged``, ``forward_ragged_pcm``, ``forward_host_ragged``, ``score_host_ragged``)
+are repeat-padded to ``max_len`` as the training loader's ``pad()`` does (maze5.py:280-285), or with ``pad="zero"``
+zero-padded as the evaluation script's dataset does (Maze5_eval.py:203-221); longer clips keep their first
+``max_len`` samples either way.
+
 The directory name carries hyphens (it mirrors the reference repository's name); import it with
 ``importlib.import_module("audio-deepfake-detection-fmsl_b200")`` or through the ``b200_frontend``
 alias module at the repository root.

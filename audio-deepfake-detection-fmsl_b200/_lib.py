@@ -20,6 +20,8 @@ ABI_VERSION = 1
 LOG_NONE, LOG_DB, LOG_LN = 0, 1, 2
 VARIANT_AUTO, VARIANT_FFT, VARIANT_DFT_GEMM = 0, 1, 2
 VARIANTS = {"auto": VARIANT_AUTO, "fft": VARIANT_FFT, "dft_gemm": VARIANT_DFT_GEMM}
+PAD_REPEAT, PAD_ZERO = 0, 1
+PAD_MODES = {"repeat": PAD_REPEAT, "zero": PAD_ZERO}
 
 OK = 0
 ERR_BAD_ARG, ERR_UNSUPPORTED, ERR_WORKSPACE, ERR_ALIGNMENT, ERR_CUDA, ERR_NO_DEVICE = -1, -2, -3, -4, -5, -6
@@ -70,6 +72,9 @@ _SIGNATURES = {
     "b200fe_spectrogram_forward": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int64, _P, C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200fe_features_forward": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, _P, C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "b200fe_features_forward_ragged_pad": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
+                                                       C.c_int32, _P, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                                       C.c_void_p]),
     "b200fe_fbank_energies_forward": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, _P,
                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "b200fe_lfcc_forward": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, _P, C.c_void_p,
@@ -86,10 +91,17 @@ _SIGNATURES = {
     "b200fe_workspace_bytes_ragged_i16": (C.c_int64, [_P, C.c_int64, C.c_int64]),
     "b200fe_features_forward_ragged_i16": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, _P,
                                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "b200fe_features_forward_ragged_i16_pad": (C.c_int32, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
+                                                           C.c_int32, _P, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                           C.c_size_t, C.c_void_p]),
     "b200fe_host_staging_bytes_ragged": (C.c_int64, [_P, C.c_int64, C.c_int64, C.c_int32, C.c_int32]),
     "b200fe_features_forward_host_ragged": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p,
                                                         C.c_int64, C.c_int64, _P, C.c_void_p, C.c_void_p, C.c_void_p,
                                                         C.c_size_t, C.c_int64, C.POINTER(C.c_void_p), C.c_int32]),
+    "b200fe_features_forward_host_ragged_pad": (C.c_int32, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p,
+                                                            C.c_int32, C.c_int64, C.c_int64, _P, C.c_void_p,
+                                                            C.c_void_p, C.c_void_p, C.c_size_t, C.c_int64,
+                                                            C.POINTER(C.c_void_p), C.c_int32]),
     "b200fe_eer_workspace_bytes": (C.c_int64, [C.c_int64]),
     "b200fe_eer_min_dcf": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "b200fe_last_launch_count": (C.c_int64, []),
@@ -118,6 +130,14 @@ def load() -> C.CDLL:
         raise OSError(f"libb200fe ABI {lib.b200fe_version()} != binding {ABI_VERSION}; rebuild")
     _lib = lib
     return lib
+
+
+def pad_mode(pad: str) -> int:
+    """``b200fe_pad_mode`` of a ragged call's ``pad`` argument: ``"repeat"`` (the training loader's ``pad()``,
+    maze5.py:280-285) or ``"zero"`` (the evaluation script's zero-padding, Maze5_eval.py:203-221)."""
+    if not isinstance(pad, str) or pad not in PAD_MODES:
+        raise ValueError(f"pad must be 'repeat' or 'zero', got {pad!r}")
+    return PAD_MODES[pad]
 
 
 def last_error() -> str:

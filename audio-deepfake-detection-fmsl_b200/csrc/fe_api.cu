@@ -178,7 +178,7 @@ extern "C" int32_t b200fe_spectrogram_forward(const float* wave, int64_t R, int6
 static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T, const int64_t* offsets,
                             const int32_t* lengths, const b200fe_params* p, const void* tables,
                             float* out, void* workspace, size_t workspace_bytes, void* stream_,
-                            bool energies_only) {
+                            bool energies_only, int32_t pad_mode) {
   const float* wave = (const float*)wave_;
   int32_t st = common_checks(p, wave_, R, T, tables, out, pcm16 ? 2 : 4);
   if (st != B200FE_OK) return st;
@@ -246,6 +246,7 @@ static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T,
   fa.radix2_first = (__builtin_ctz(p->n_fft / 2) & 1);
   fa.top_db_group = p->top_db_group;
   fa.preemph = p->preemph;
+  fa.pad_zero = pad_mode == B200FE_PAD_ZERO;
   if (variant == B200FE_VARIANT_FFT) {
     fa.ft = fe_fft_pick_ft(p->n_fft, p->hop_length, p->n_filter, 1);
     if (fa.ft == 0) { fe_set_error("n_fft=%d hop=%d does not fit shared memory", p->n_fft, p->hop_length); return B200FE_ERR_UNSUPPORTED; }
@@ -299,8 +300,10 @@ static int32_t run_features(const void* wave_, bool pcm16, int64_t R, int64_t T,
           dense_rel = dr;
         }
       }
-      e = pcm16 ? fe_launch_dense_rows((const int16_t*)wave_, offsets, lengths, r0, nr, T, p->preemph, dense, stream)
-                : fe_launch_dense_rows(wave, offsets, lengths, r0, nr, T, p->preemph, dense, stream, flat_rel);
+      e = pcm16 ? fe_launch_dense_rows((const int16_t*)wave_, offsets, lengths, r0, nr, T, p->preemph, dense, stream, 0,
+                                       fa.pad_zero)
+                : fe_launch_dense_rows(wave, offsets, lengths, r0, nr, T, p->preemph, dense, stream, flat_rel, 0,
+                                       fa.pad_zero);
       if (e != cudaSuccess) return cuda_fail(e, "dense-rows kernel launch");
       fs.wave_chunk = dense;
       fs.preemph = 0.0f;
@@ -338,21 +341,55 @@ extern "C" int32_t b200fe_features_forward(const float* wave, int64_t R, int64_t
                                            const int32_t* lengths, const b200fe_params* p, const void* tables,
                                            float* out, void* workspace, size_t workspace_bytes, void* stream) {
   fe_launch_count = 0;
-  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
+  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false,
+                      B200FE_PAD_REPEAT);
 }
 
 extern "C" int32_t b200fe_features_forward_ragged_i16(const int16_t* pcm, int64_t R, int64_t T, const int64_t* offsets,
                                                       const int32_t* lengths, const b200fe_params* p, const void* tables,
                                                       float* out, void* workspace, size_t workspace_bytes, void* stream) {
   fe_launch_count = 0;
-  return run_features(pcm, true, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
+  return run_features(pcm, true, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false,
+                      B200FE_PAD_REPEAT);
+}
+
+// The pad_mode argument of the *_pad entry points, checked before any CUDA call.
+static int32_t check_pad_mode(int32_t pad_mode) {
+  if (pad_mode == B200FE_PAD_REPEAT || pad_mode == B200FE_PAD_ZERO) return B200FE_OK;
+  fe_set_error("pad_mode=%d must be B200FE_PAD_REPEAT (0) or B200FE_PAD_ZERO (1)", pad_mode);
+  return B200FE_ERR_BAD_ARG;
+}
+
+extern "C" int32_t b200fe_features_forward_ragged_pad(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
+                                                      const int32_t* lengths, int32_t pad_mode, const b200fe_params* p,
+                                                      const void* tables, float* out, void* workspace,
+                                                      size_t workspace_bytes, void* stream) {
+  fe_launch_count = 0;
+  const int32_t st = check_pad_mode(pad_mode);
+  if (st != B200FE_OK) return st;
+  if (!offsets || !lengths) { fe_set_error("offsets / lengths is NULL"); return B200FE_ERR_BAD_ARG; }
+  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false,
+                      pad_mode);
+}
+
+extern "C" int32_t b200fe_features_forward_ragged_i16_pad(const int16_t* pcm, int64_t R, int64_t T,
+                                                          const int64_t* offsets, const int32_t* lengths,
+                                                          int32_t pad_mode, const b200fe_params* p, const void* tables,
+                                                          float* out, void* workspace, size_t workspace_bytes,
+                                                          void* stream) {
+  fe_launch_count = 0;
+  const int32_t st = check_pad_mode(pad_mode);
+  if (st != B200FE_OK) return st;
+  return run_features(pcm, true, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false,
+                      pad_mode);
 }
 
 extern "C" int32_t b200fe_fbank_energies_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
                                                  const int32_t* lengths, const b200fe_params* p, const void* tables,
                                                  float* out, void* workspace, size_t workspace_bytes, void* stream) {
   fe_launch_count = 0;
-  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, true);
+  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, true,
+                      B200FE_PAD_REPEAT);
 }
 
 extern "C" int32_t b200fe_lfcc_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
@@ -360,7 +397,8 @@ extern "C" int32_t b200fe_lfcc_forward(const float* wave, int64_t R, int64_t T, 
                                        float* out, void* workspace, size_t workspace_bytes, void* stream) {
   fe_launch_count = 0;
   if (p && p->n_coef < 1) { fe_set_error("b200fe_lfcc_forward needs n_coef >= 1"); return B200FE_ERR_BAD_ARG; }
-  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
+  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false,
+                      B200FE_PAD_REPEAT);
 }
 
 extern "C" int32_t b200fe_mel_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
@@ -368,7 +406,8 @@ extern "C" int32_t b200fe_mel_forward(const float* wave, int64_t R, int64_t T, c
                                       float* out, void* workspace, size_t workspace_bytes, void* stream) {
   fe_launch_count = 0;
   if (p && p->n_coef != 0) { fe_set_error("b200fe_mel_forward needs n_coef == 0"); return B200FE_ERR_BAD_ARG; }
-  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false);
+  return run_features(wave, false, R, T, offsets, lengths, p, tables, out, workspace, workspace_bytes, stream, false,
+                      B200FE_PAD_REPEAT);
 }
 
 extern "C" int32_t b200fe_compute_deltas(const float* in, int64_t rows, int64_t T, int32_t win, float* out,
@@ -490,11 +529,11 @@ int64_t ragged_chunk(const host_input& in, int64_t r0, int64_t max_rows, int64_t
 //   dense float32: H2D rows -> dense forward -> D2H features
 //   dense 16-bit PCM: H2D rows -> stage float32 rows (x / 32768, pre-emphasis) -> dense forward without pre-emphasis
 //                     -> D2H features
-//   ragged: H2D copy span, H2D clip table slice -> stage float32 rows (pad(), x / 32768, pre-emphasis) -> dense forward
-//           without pre-emphasis -> D2H features
+//   ragged: H2D copy span, H2D clip table slice -> stage float32 rows (pad() or zero-padding as pad_mode says,
+//           x / 32768, pre-emphasis) -> dense forward without pre-emphasis -> D2H features
 int32_t forward_host(const host_input& in, int64_t R, int64_t T, const b200fe_params* p, const void* tables,
                      float* out_host, void* staging, size_t staging_bytes, int64_t chunk_rows, void* const* streams,
-                     int32_t n_streams) {
+                     int32_t n_streams, int32_t pad_mode) {
   const bool ragged = in.offsets != nullptr;
   if (!in.data || !out_host || !staging || !streams || !p) { fe_set_error("NULL argument"); return B200FE_ERR_BAD_ARG; }
   if (R < 1) { fe_set_error("R=%lld must be >= 1", (long long)R); return B200FE_ERR_BAD_ARG; }
@@ -521,6 +560,7 @@ int32_t forward_host(const host_input& in, int64_t R, int64_t T, const b200fe_pa
   const size_t in_elt = (size_t)in.sample_bytes;
   const bool pcm16 = in.sample_bytes == 2;
   const int64_t span_cap = chunk_rows * (T + kSpanSlack);
+  const int pad_zero = pad_mode == B200FE_PAD_ZERO;
   int64_t c = 0;
   for (int64_t r0 = 0; r0 < R; ++c) {
     const int64_t max_rows = R - r0 < chunk_rows ? R - r0 : chunk_rows;
@@ -554,12 +594,13 @@ int32_t forward_host(const host_input& in, int64_t R, int64_t T, const b200fe_pa
       if (e != cudaSuccess) return cuda_fail(e, "H2D copy (lengths)");
     }
     if (ragged || pcm16) {
-      e = pcm16 ? fe_launch_dense_rows((const int16_t*)d_in, d_off, d_len, 0, nr, T, p->preemph, d_wave, st, lo)
-                : fe_launch_dense_rows((const float*)d_in, d_off, d_len, 0, nr, T, p->preemph, d_wave, st, -1, lo);
+      e = pcm16 ? fe_launch_dense_rows((const int16_t*)d_in, d_off, d_len, 0, nr, T, p->preemph, d_wave, st, lo, pad_zero)
+                : fe_launch_dense_rows((const float*)d_in, d_off, d_len, 0, nr, T, p->preemph, d_wave, st, -1, lo,
+                                       pad_zero);
       if (e != cudaSuccess) return cuda_fail(e, "dense-rows kernel launch");
     }
     int32_t rc = run_features(d_wave, false, nr, T, nullptr, nullptr, &q, tables, d_out, d_ws, (size_t)L.ws_bytes, st,
-                              false);
+                              false, B200FE_PAD_REPEAT);
     if (rc != B200FE_OK) return rc;
     e = cudaMemcpyAsync(out_host + (size_t)r0 * n_out * nf, d_out, (size_t)nr * n_out * nf * 4, cudaMemcpyDeviceToHost, st);
     if (e != cudaSuccess) return cuda_fail(e, "D2H copy");
@@ -594,7 +635,7 @@ extern "C" int32_t b200fe_features_forward_host(const float* wave_host, int64_t 
                                                 int32_t n_streams) {
   fe_launch_count = 0;
   return forward_host(dense_input(wave_host, 4), R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams,
-                      n_streams);
+                      n_streams, B200FE_PAD_REPEAT);
 }
 
 extern "C" int32_t b200fe_features_forward_host_i16(const int16_t* pcm_host, int64_t R, int64_t T, const b200fe_params* p,
@@ -603,7 +644,7 @@ extern "C" int32_t b200fe_features_forward_host_i16(const int16_t* pcm_host, int
                                                     int32_t n_streams) {
   fe_launch_count = 0;
   return forward_host(dense_input(pcm_host, 2), R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams,
-                      n_streams);
+                      n_streams, B200FE_PAD_REPEAT);
 }
 
 extern "C" int32_t b200fe_features_forward_host_ragged(const void* clips_host, int32_t sample_bytes, int64_t n_samples,
@@ -611,9 +652,23 @@ extern "C" int32_t b200fe_features_forward_host_ragged(const void* clips_host, i
                                                        int64_t R, int64_t T, const b200fe_params* p, const void* tables,
                                                        float* out_host, void* staging, size_t staging_bytes,
                                                        int64_t chunk_rows, void* const* streams, int32_t n_streams) {
+  return b200fe_features_forward_host_ragged_pad(clips_host, sample_bytes, n_samples, offsets_host, lengths_host,
+                                                 B200FE_PAD_REPEAT, R, T, p, tables, out_host, staging, staging_bytes,
+                                                 chunk_rows, streams, n_streams);
+}
+
+extern "C" int32_t b200fe_features_forward_host_ragged_pad(const void* clips_host, int32_t sample_bytes,
+                                                           int64_t n_samples, const int64_t* offsets_host,
+                                                           const int32_t* lengths_host, int32_t pad_mode, int64_t R,
+                                                           int64_t T, const b200fe_params* p, const void* tables,
+                                                           float* out_host, void* staging, size_t staging_bytes,
+                                                           int64_t chunk_rows, void* const* streams,
+                                                           int32_t n_streams) {
   fe_launch_count = 0;
+  const int32_t st = check_pad_mode(pad_mode);
+  if (st != B200FE_OK) return st;
   if (!offsets_host || !lengths_host) { fe_set_error("offsets / lengths is NULL"); return B200FE_ERR_BAD_ARG; }
   if (n_samples < 1) { fe_set_error("n_samples=%lld must be >= 1", (long long)n_samples); return B200FE_ERR_BAD_ARG; }
   const host_input in{clips_host, sample_bytes, offsets_host, lengths_host, n_samples};
-  return forward_host(in, R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams, n_streams);
+  return forward_host(in, R, T, p, tables, out_host, staging, staging_bytes, chunk_rows, streams, n_streams, pad_mode);
 }

@@ -128,27 +128,30 @@ FE_HD int fe_reflect_index(int pp, int half, int T) {
 // Staging phase: thread `tid` of `nthreads` fills s_stage[i] for padded positions pp0 + i, i < seg.
 // Padding is torch.stft's reflect padding by n_fft/2; the T-sample signal is the clip repeat-padded
 // or truncated to T (pad(), Thesis/01_Models/01_Baseline_Models/maze5.py:280-285: sample r =
-// clip[r mod len]); optional pre-emphasis y[r] = x[r] - a*x[r-1], y[0] = x[0]
-// (torchaudio functional/functional.py:2426-2448) is applied before the padding, as torchaudio would.
-// Sample r (0 <= r < T) of the T-sample signal a clip stands for: repeat-pad / truncate, then pre-emphasis.
-FE_HD float fe_padded_sample(const float* src, int clip_len, int T, int r, float preemph) {
-  const bool wrap = clip_len < T;
+// clip[r mod len]), or with pad_zero != 0 zero-padded or truncated to T (the evaluation script's
+// dataset: sample r = clip[r] for r < len, 0 after); optional pre-emphasis y[r] = x[r] - a*x[r-1],
+// y[0] = x[0] (torchaudio functional/functional.py:2426-2448) is applied to the T-sample signal
+// before the reflect padding, as torchaudio would.
+// Sample r (0 <= r < T) of the T-sample signal a clip stands for: pad / truncate, then pre-emphasis.
+// Without wrap-around every index c < T, so c >= clip_len happens only past the end of a zero-padded clip.
+FE_HD float fe_padded_sample(const float* src, int clip_len, int T, int r, float preemph, int pad_zero = 0) {
+  const bool wrap = clip_len < T && !pad_zero;
   const int c = wrap ? (r % clip_len) : r;
-  float v = src[c];
+  float v = c < clip_len ? src[c] : 0.0f;
   if (preemph != 0.0f && r > 0) {
     const int c1 = wrap ? ((r - 1) % clip_len) : (r - 1);
-    v = fmaf(-preemph, src[c1], v);
+    v = fmaf(-preemph, c1 < clip_len ? src[c1] : 0.0f, v);
   }
   return v;
 }
 
 FE_HD void fe_stage_load(int tid, int nthreads, const float* src, int clip_len, int T, int n_fft, int pp0,
-                         int seg, float preemph, float* s_stage) {
+                         int seg, float preemph, float* s_stage, int pad_zero = 0) {
   const int half = n_fft >> 1;
 #pragma unroll 4
   for (int i = tid; i < seg; i += nthreads) {
     const int r = fe_reflect_index(pp0 + i, half, T);
-    s_stage[i] = fe_padded_sample(src, clip_len, T, r, preemph);
+    s_stage[i] = fe_padded_sample(src, clip_len, T, r, preemph, pad_zero);
   }
 }
 

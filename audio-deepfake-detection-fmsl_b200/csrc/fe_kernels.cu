@@ -207,7 +207,8 @@ __global__ void __launch_bounds__(kFftThreads) fe_fft_kernel(fe_fft_args a) {
 
   // ---- stage the waveform segment -------------------------------------------------------------
   // Padded position pp = t0*hop + i  (reflect padding by n_fft/2, torch.stft center=True); the
-  // T-sample signal itself is the clip repeat-padded / truncated to T (pad(), maze5.py:280-285).
+  // T-sample signal itself is the clip repeat-padded (pad(), maze5.py:280-285) or zero-padded (a.pad_zero) /
+  // truncated to T.
   {
     const float* src;
     int clip_len;  // T < 2^31 is checked on the host
@@ -219,7 +220,7 @@ __global__ void __launch_bounds__(kFftThreads) fe_fft_kernel(fe_fft_args a) {
       clip_len = (int)a.T;
     }
     const int seg_here = (nf_here - 1) * hop + n_fft;
-    fe_stage_load(tid, kFftThreads, src, clip_len, (int)a.T, n_fft, t0 * hop, seg_here, a.preemph, s_stage);
+    fe_stage_load(tid, kFftThreads, src, clip_len, (int)a.T, n_fft, t0 * hop, seg_here, a.preemph, s_stage, a.pad_zero);
   }
   __syncthreads();
 
@@ -426,7 +427,8 @@ __global__ void __launch_bounds__(kFftThreads, E == 16 ? 2 : 4) fe_rfft_kernel(f
       return true;
     }
     if (async_only) return false;
-    fe_stage_load(tid, kFftThreads, src, clip_len, (int)a.T, NFFT, t0_b * hop, seg_here, a.preemph, s_stage);
+    fe_stage_load(tid, kFftThreads, src, clip_len, (int)a.T, NFFT, t0_b * hop, seg_here, a.preemph, s_stage,
+                  a.pad_zero);
     return true;
   };
   bool prefetched = false;
@@ -930,8 +932,9 @@ __global__ void fe_deltas_kernel(const float* __restrict__ in, float* __restrict
 }
 
 // ------------------------------------------------------------------------------------------------
-// fe_dense_rows_kernel : clips (ragged, repeat-padded / truncated to T as pad() does, maze5.py:280-285)
-// and / or pre-emphasis -> dense rows [rows][T] the streaming tcgen05 kernel can fetch with TMA boxes.
+// fe_dense_rows_kernel : clips (ragged, repeat-padded / truncated to T as pad() does, maze5.py:280-285, or zero-padded /
+// truncated with pad_zero) and / or pre-emphasis -> dense rows [rows][T] the streaming tcgen05 kernel can fetch with
+// TMA boxes.
 // One thread = four consecutive samples of one row, one 16-byte store (VEC4: T % 4 == 0; otherwise four scalar stores,
 // for the FFT variant, which reads dense rows of any T).  Samples are float32 or 16-bit PCM converted as x / 32768
 // (exact in fp32: what a FLAC / WAV decoder's float conversion yields), read one at a time: an int16 clip may start on
@@ -946,7 +949,7 @@ __global__ void __launch_bounds__(256) fe_dense_rows_kernel(const S* __restrict_
                                                            const int64_t* __restrict__ offsets,
                                                            const int32_t* __restrict__ lengths, int64_t row_base,
                                                            int T, float preemph, float* __restrict__ dst,
-                                                           int64_t flat_rel, int64_t base) {
+                                                           int64_t flat_rel, int64_t base, int pad_zero) {
   const int64_t row = row_base + blockIdx.y;
   const S* src;
   int clip_len;
@@ -960,17 +963,31 @@ __global__ void __launch_bounds__(256) fe_dense_rows_kernel(const S* __restrict_
   }
   float* d = dst + (int64_t)blockIdx.y * T;
   // same values as fe_padded_sample(), with the clip index carried instead of recomputed per sample
+  const bool wrap = clip_len < T && !pad_zero;
+  const bool zero_tail = clip_len < T && pad_zero;
   for (int r = (blockIdx.x * blockDim.x + threadIdx.x) * 4; r < T; r += gridDim.x * blockDim.x * 4) {
-    int c = clip_len < T ? r % clip_len : r;
+    if (zero_tail && r > clip_len) {   // past the clip and its pre-emphasis boundary y[len]: zeros, nothing to read
+      if (VEC4) {
+        *reinterpret_cast<float4*>(d + r) = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+      } else {
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+          if (r + i < T) d[r + i] = 0.0f;
+      }
+      continue;
+    }
+    // wrap: c < clip_len.  Otherwise c = r + i, which reaches clip_len only in a zero tail (samples 0, and `prev`
+    // carries clip[len-1] into y[len])
+    int c = wrap ? r % clip_len : r;
     float prev = 0.0f;
     if (preemph != 0.0f && r > 0) prev = fe_sample_f32(src[c == 0 ? clip_len - 1 : c - 1]);
     float v[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-      const float x = (VEC4 || r + i < T) ? fe_sample_f32(src[c]) : 0.0f;
+      const float x = ((VEC4 || r + i < T) && c < clip_len) ? fe_sample_f32(src[c]) : 0.0f;
       v[i] = (preemph != 0.0f && r + i > 0) ? fmaf(-preemph, prev, x) : x;
       prev = x;
-      c = (c + 1 == clip_len && clip_len < T) ? 0 : c + 1;
+      c = (c + 1 == clip_len && wrap) ? 0 : c + 1;
     }
     if (VEC4) {
       *reinterpret_cast<float4*>(d + r) = make_float4(v[0], v[1], v[2], v[3]);
@@ -1288,7 +1305,7 @@ cudaError_t fe_launch_deltas(const float* in, float* out, int64_t rows, int64_t 
 template <typename S>
 static cudaError_t launch_dense_rows(const S* wave, const int64_t* offsets, const int32_t* lengths, int64_t row_base,
                                      int64_t rows, int64_t T, float preemph, float* dst, cudaStream_t stream,
-                                     int64_t flat_rel, int64_t base) {
+                                     int64_t flat_rel, int64_t base, int pad_zero) {
   // CTAs per row: each thread walks its row in T / (1024 bx) steps.  One CTA per 1024 samples (64 per LFCC row) was
   // measured slowest; 16 per row is best when every row is copied (all-staged ragged step 1.30 -> 1.24 ms per 4096
   // clips, profiles/r2_ragged_inplace.txt), 8 when rows the streaming kernel reads in place are in the batch: those
@@ -1301,22 +1318,23 @@ static cudaError_t launch_dense_rows(const S* wave, const int64_t* offsets, cons
     dim3 grid(bx, (unsigned)nr);
     if (vec4)
       fe_dense_rows_kernel<S, true><<<grid, 256, 0, stream>>>(wave, offsets, lengths, row_base + r0, (int)T, preemph,
-                                                              dst + r0 * T, flat_rel, base);
+                                                              dst + r0 * T, flat_rel, base, pad_zero);
     else
       fe_dense_rows_kernel<S, false><<<grid, 256, 0, stream>>>(wave, offsets, lengths, row_base + r0, (int)T, preemph,
-                                                               dst + r0 * T, flat_rel, base);
+                                                               dst + r0 * T, flat_rel, base, pad_zero);
     return cudaSuccess;
   });
 }
 
 cudaError_t fe_launch_dense_rows(const float* wave, const int64_t* offsets, const int32_t* lengths,
                                  int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
-                                 cudaStream_t stream, int64_t flat_rel, int64_t base) {
-  return launch_dense_rows(wave, offsets, lengths, row_base, rows, T, preemph, dst, stream, flat_rel, base);
+                                 cudaStream_t stream, int64_t flat_rel, int64_t base, int pad_zero) {
+  return launch_dense_rows(wave, offsets, lengths, row_base, rows, T, preemph, dst, stream, flat_rel, base, pad_zero);
 }
 
 cudaError_t fe_launch_dense_rows(const int16_t* wave, const int64_t* offsets, const int32_t* lengths,
                                  int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
-                                 cudaStream_t stream, int64_t base) {
-  return launch_dense_rows(wave, offsets, lengths, row_base, rows, T, preemph, dst, stream, (int64_t)-1, base);
+                                 cudaStream_t stream, int64_t base, int pad_zero) {
+  return launch_dense_rows(wave, offsets, lengths, row_base, rows, T, preemph, dst, stream, (int64_t)-1, base,
+                           pad_zero);
 }

@@ -27,6 +27,7 @@ struct fe_fft_args {
   int32_t fft_warps;        // warps that own FFT buffers (set by fe_launch_fft)
   int32_t top_db_group;
   float preemph;
+  int32_t pad_zero;         // ragged clips read through fe_stage_load: 1 = zero-pad short clips, 0 = repeat-pad
 };
 
 struct fe_tail_args {
@@ -89,14 +90,15 @@ cudaError_t fe_launch_tail(const fe_tail_args& a, int64_t rows, cudaStream_t str
 cudaError_t fe_launch_cmvn(float* out, int64_t n_series, int n_frames, cudaStream_t stream);
 cudaError_t fe_launch_deltas(const float* in, float* out, int64_t rows, int64_t T, int win,
                              cudaStream_t stream);
-// Dense [rows][T] copy of rows [row_base, row_base+rows): repeat-pad / truncate ragged clips and apply
-// pre-emphasis, so the streaming kernel (TMA boxes over dense rows) serves those inputs too.  dst 16-byte aligned.
-// Ragged row r reads its clip at wave + offsets[r] - base (`wave` may hold only a span of the flat buffer).
+// Dense [rows][T] copy of rows [row_base, row_base+rows): repeat-pad (pad_zero 0) or zero-pad (pad_zero 1) / truncate
+// ragged clips and apply pre-emphasis, so the streaming kernel (TMA boxes over dense rows) serves those inputs too.
+// dst 16-byte aligned.  Ragged row r reads its clip at wave + offsets[r] - base (`wave` may hold only a span of the
+// flat buffer).
 cudaError_t fe_launch_dense_rows(const float* wave, const int64_t* offsets, const int32_t* lengths,
                                  int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
-                                 cudaStream_t stream, int64_t flat_rel = -1, int64_t base = 0);
+                                 cudaStream_t stream, int64_t flat_rel = -1, int64_t base = 0, int pad_zero = 0);
 // The same from 16-bit PCM (x / 32768, exact); every row is written (no clip is read in place).
 cudaError_t fe_launch_dense_rows(const int16_t* wave, const int64_t* offsets, const int32_t* lengths,
                                  int64_t row_base, int64_t rows, int64_t T, float preemph, float* dst,
-                                 cudaStream_t stream, int64_t base = 0);
+                                 cudaStream_t stream, int64_t base = 0, int pad_zero = 0);
 #endif

@@ -22,6 +22,7 @@ import torch
 import torch.distributed as dist
 from torch import Tensor, nn
 
+from . import _lib
 from .evaluation import eer_min_dcf, eer_min_dcf_device, gather_scores, shard_range
 
 N_BONAFIDE, N_SPOOF = 7355, 63882          # Eval.py:58-60
@@ -181,7 +182,7 @@ def score_host_pcm(frontend: nn.Module, scorer: nn.Module, pcm_host: Tensor, dev
 
 def score_host_ragged(frontend: nn.Module, scorer: nn.Module, flat_host: Tensor, offsets: Tensor, lengths: Tensor,
                       device: torch.device, *, max_len: int = UTT_LEN, chunk_rows: int = 1024, n_streams: int = 2,
-                      out_host: Optional[Tensor] = None) -> Tensor:
+                      out_host: Optional[Tensor] = None, pad: str = "repeat") -> Tensor:
     """``score_host_pcm`` for variable-length clips in HOST memory (maze5.py:297-351 loader and :280-285 ``pad()`` ->
     :415-430 scoring loop): a flat int16 PCM or float32 CPU buffer (pinned for asynchronous copies) and its int64
     ``offsets`` / int32 ``lengths`` clip table.  The table is checked once on the host; then each chunk of
@@ -189,7 +190,10 @@ def score_host_ragged(frontend: nn.Module, scorer: nn.Module, flat_host: Tensor,
     ``pad()`` reads) and its offsets rebased to that span on its own stream, and runs ``frontend.forward_ragged_pcm``
     (int16) or ``frontend.forward_ragged`` (float32) and the classifier there.  Features stay on the device; returns
     the bonafide scores ``float32[R]`` on the host (pinned), those of ``scorer(frontend.forward_ragged(...))`` on the
-    same chunks."""
+    same chunks.  ``pad="repeat"`` tiles clips shorter than ``max_len`` as the training loader's ``pad()`` does;
+    ``pad="zero"`` appends zeros, as the evaluation script's dataset does (Maze5_eval.py:203-221), for the scores (and
+    then the EER) that script computes."""
+    _lib.pad_mode(pad)                            # ValueError before anything is copied or launched
     if flat_host.device.type != "cpu" or flat_host.dim() != 1 or flat_host.dtype not in (torch.int16, torch.float32):
         raise TypeError("score_host_ragged expects a 1-D int16 (16-bit PCM) or float32 CPU tensor")
     if offsets.dtype != torch.int64 or lengths.dtype != torch.int32:
@@ -230,7 +234,7 @@ def score_host_ragged(frontend: nn.Module, scorer: nn.Module, flat_host: Tensor,
             d_off = rebased[r0:r1].to(device, non_blocking=True)
             d_len = lengths_pinned[r0:r1].to(device, non_blocking=True)
             fwd = frontend.forward_ragged_pcm if pcm16 else frontend.forward_ragged
-            feats = fwd(d, d_off, d_len, max_len=T, validate=False)
+            feats = fwd(d, d_off, d_len, max_len=T, validate=False, pad=pad)
             scores[r0:r1] = scorer(feats)[:, 1]                       # maze5.py:425
     for s in streams:
         cur.wait_stream(s)

@@ -295,12 +295,18 @@ class FrontEndEngine:
 
     def features(self, wave2d: Tensor, group: int = 1, out: Optional[Tensor] = None,
                  offsets: Optional[Tensor] = None, lengths: Optional[Tensor] = None,
-                 T: Optional[int] = None, validate: bool = True) -> Tensor:
+                 T: Optional[int] = None, validate: bool = True, *, pad: str = "repeat") -> Tensor:
         """``wave2d`` is ``(R,T)`` contiguous, or — with ``offsets``/``lengths``/``T`` — the flat
         ragged clip buffer.  Returns ``(R, n_out, n_frames)``.  ``validate`` (ragged input only) checks the
         clip table on the device first — every clip non-empty and inside the flat buffer, as the
         reference's ``pad()`` would raise on an empty clip (maze5.py:280-285); it costs one host
-        synchronisation per call and can be switched off by callers that built the table themselves."""
+        synchronisation per call and can be switched off by callers that built the table themselves.
+        ``pad`` (ragged input only) says how a clip shorter than ``T`` is filled: ``"repeat"`` tiles it as the
+        training loader's ``pad()`` does, ``"zero"`` appends zeros as the evaluation script's dataset does
+        (Maze5_eval.py:203-221); a longer clip keeps its first ``T`` samples either way."""
+        pad_mode = _lib.pad_mode(pad)
+        if offsets is None and pad_mode != _lib.PAD_REPEAT:
+            raise ValueError("pad applies to ragged input (offsets / lengths) only")
         self._check_wave(wave2d)
         dev = wave2d.device
         if offsets is None:
@@ -325,12 +331,14 @@ class FrontEndEngine:
             stream = torch.cuda.current_stream(dev).cuda_stream
             with self._lock:
                 ws = self.workspace_on(dev, ws_bytes, stream)
-                _lib.check(self.lib.b200fe_features_forward(
-                    wave2d.data_ptr(), R, T,
-                    None if offsets is None else offsets.data_ptr(),
-                    None if lengths is None else lengths.data_ptr(),
-                    C.byref(p), self.tables_on(dev).data_ptr(), out.data_ptr(), ws.data_ptr(), ws.numel(),
-                    C.c_void_p(stream)))
+                if offsets is None:
+                    _lib.check(self.lib.b200fe_features_forward(
+                        wave2d.data_ptr(), R, T, None, None, C.byref(p), self.tables_on(dev).data_ptr(),
+                        out.data_ptr(), ws.data_ptr(), ws.numel(), C.c_void_p(stream)))
+                else:
+                    _lib.check(self.lib.b200fe_features_forward_ragged_pad(
+                        wave2d.data_ptr(), R, T, offsets.data_ptr(), lengths.data_ptr(), pad_mode, C.byref(p),
+                        self.tables_on(dev).data_ptr(), out.data_ptr(), ws.data_ptr(), ws.numel(), C.c_void_p(stream)))
         if torch.cuda.current_device() == (dev.index if dev.index is not None else torch.cuda.current_device()):
             launch()                       # (the device guard costs a few microseconds per call)
         else:
@@ -339,10 +347,12 @@ class FrontEndEngine:
         return out
 
     def features_ragged_pcm(self, flat_i16: Tensor, offsets: Tensor, lengths: Tensor, T: int,
-                            out: Optional[Tensor] = None, validate: bool = True) -> Tensor:
-        """The ragged call of ``features`` with 16-bit PCM clips on the device (``b200fe_features_forward_ragged_i16``):
-        every row is staged as a dense float32 row, ``x / 32768`` (exact), so the features are those of the float32
-        ragged call on ``flat_i16.float() / 32768``, bit for bit.  Returns ``(R, n_out, n_frames)``."""
+                            out: Optional[Tensor] = None, validate: bool = True, *, pad: str = "repeat") -> Tensor:
+        """The ragged call of ``features`` with 16-bit PCM clips on the device
+        (``b200fe_features_forward_ragged_i16_pad``): every row is staged as a dense float32 row, ``x / 32768`` (exact),
+        so the features are those of the float32 ragged call on ``flat_i16.float() / 32768`` with the same ``pad``,
+        bit for bit.  Returns ``(R, n_out, n_frames)``."""
+        pad_mode = _lib.pad_mode(pad)
         if not isinstance(flat_i16, Tensor) or flat_i16.dtype != torch.int16:
             raise TypeError(f"features_ragged_pcm expects int16 PCM, got "
                             f"{flat_i16.dtype if isinstance(flat_i16, Tensor) else type(flat_i16)}")
@@ -365,8 +375,8 @@ class FrontEndEngine:
         with torch.cuda.device(dev), self._lock:
             stream = torch.cuda.current_stream(dev).cuda_stream
             ws = self.workspace_on(dev, ws_bytes, stream)
-            _lib.check(self.lib.b200fe_features_forward_ragged_i16(
-                flat_i16.data_ptr(), R, T, offsets.data_ptr(), lengths.data_ptr(), C.byref(p),
+            _lib.check(self.lib.b200fe_features_forward_ragged_i16_pad(
+                flat_i16.data_ptr(), R, T, offsets.data_ptr(), lengths.data_ptr(), pad_mode, C.byref(p),
                 self.tables_on(dev).data_ptr(), out.data_ptr(), ws.data_ptr(), ws.numel(), C.c_void_p(stream)))
         return out
 
@@ -433,14 +443,16 @@ class FrontEndEngine:
 
     def features_host_ragged(self, flat_host: Tensor, offsets_host: Tensor, lengths_host: Tensor, T: int,
                              out_host: Optional[Tensor] = None, *, device=None, chunk_rows: int = 512,
-                             n_streams: int = 3) -> Tensor:
-        """End-to-end path for variable-length clips in HOST memory (``b200fe_features_forward_host_ragged``): a flat
-        float32 or int16 PCM CPU buffer (ideally pinned) with an int64 ``offsets`` / int32 ``lengths`` clip table in,
-        HOST features ``(R, n_out, n_frames)`` out, each clip repeat-padded / truncated to ``T`` as ``pad()`` does.
+                             n_streams: int = 3, pad: str = "repeat") -> Tensor:
+        """End-to-end path for variable-length clips in HOST memory (``b200fe_features_forward_host_ragged_pad``): a
+        flat float32 or int16 PCM CPU buffer (ideally pinned) with an int64 ``offsets`` / int32 ``lengths`` clip table
+        in, HOST features ``(R, n_out, n_frames)`` out, each clip repeat-padded / truncated to ``T`` as ``pad()`` does
+        (``pad="repeat"``) or zero-padded / truncated (``pad="zero"``, see ``features``).
         Only the samples ``pad()`` reads of each chunk's span cross PCIe (pack with ``pack_clips(max_len=T)`` to keep
         the spans tight); the rows are staged on the device.  The clip table is checked on the host (``ValueError``).
         Features are those of ``features`` / ``features_ragged_pcm`` on the same clips, bit for bit.  Shares the staging
         buffer, copy streams and lock of ``features_host``."""
+        pad_mode = _lib.pad_mode(pad)
         if not isinstance(flat_host, Tensor) or flat_host.device.type != "cpu" or flat_host.dim() != 1 \
                 or flat_host.dtype not in (torch.float32, torch.int16):
             raise TypeError("features_host_ragged expects a 1-D float32 (or int16 PCM) CPU tensor")
@@ -467,9 +479,9 @@ class FrontEndEngine:
         n_streams = max(1, min(int(n_streams), 4))
         p = self._params_for_call(self.params, T, None, True)   # every row is staged (256-byte aligned)
         need = _lib.check(self.lib.b200fe_host_staging_bytes_ragged(C.byref(p), chunk_rows, T, sample_bytes, n_streams))
-        self._host_call(device, need, n_streams, lambda tables, st, arr: self.lib.b200fe_features_forward_host_ragged(
+        self._host_call(device, need, n_streams, lambda tables, st, arr: self.lib.b200fe_features_forward_host_ragged_pad(
             flat_host.data_ptr(), sample_bytes, flat_host.numel(), offsets_host.data_ptr(), lengths_host.data_ptr(),
-            R, T, C.byref(p), tables.data_ptr(), out_host.data_ptr(), st.data_ptr(), st.numel(), chunk_rows, arr,
+            pad_mode, R, T, C.byref(p), tables.data_ptr(), out_host.data_ptr(), st.data_ptr(), st.numel(), chunk_rows, arr,
             n_streams))
         return out_host
 
@@ -573,27 +585,29 @@ class _Base(nn.Module):
         return out.reshape(shape[:-1] + out.shape[-2:])
 
     def forward_ragged(self, flat: Tensor, offsets: Tensor, lengths: Tensor, max_len: int = 64600,
-                       validate: bool = True) -> Tensor:
+                       validate: bool = True, *, pad: str = "repeat") -> Tensor:
         """Config-5 entry: ``flat`` holds variable-length clips back to back; clip ``r`` is
         ``flat[offsets[r] : offsets[r] + lengths[r]]`` and is repeat-padded / truncated to ``max_len``
-        inside the loader exactly like ``pad()`` (maze5.py:280-285).  Returns ``(R, C, n_frames)``."""
-        return self.engine.features(flat, group=1, offsets=offsets, lengths=lengths, T=int(max_len), validate=validate)
+        inside the loader exactly like ``pad()`` (maze5.py:280-285), or with ``pad="zero"`` zero-padded / truncated
+        as the evaluation script's dataset does (Maze5_eval.py:203-221).  Returns ``(R, C, n_frames)``."""
+        return self.engine.features(flat, group=1, offsets=offsets, lengths=lengths, T=int(max_len), validate=validate,
+                                    pad=pad)
 
     def forward_ragged_pcm(self, flat: Tensor, offsets: Tensor, lengths: Tensor, max_len: int = 64600,
-                           validate: bool = True) -> Tensor:
+                           validate: bool = True, *, pad: str = "repeat") -> Tensor:
         """``forward_ragged`` for 16-bit PCM clips on the device (``flat`` int16, converted ``x / 32768`` while the rows
-        are staged): the features of ``forward_ragged(flat.float() / 32768, ...)``, bit for bit."""
-        return self.engine.features_ragged_pcm(flat, offsets, lengths, int(max_len), validate=validate)
+        are staged): the features of ``forward_ragged(flat.float() / 32768, ..., pad=pad)``, bit for bit."""
+        return self.engine.features_ragged_pcm(flat, offsets, lengths, int(max_len), validate=validate, pad=pad)
 
     def forward_host(self, wave_host: Tensor, out_host: Optional[Tensor] = None, **kw) -> Tensor:
         """Host in / host out with pipelined copies (see ``FrontEndEngine.features_host``)."""
         return self.engine.features_host(wave_host, out_host, **kw)
 
     def forward_host_ragged(self, flat_host: Tensor, offsets: Tensor, lengths: Tensor, max_len: int = 64600,
-                            out_host: Optional[Tensor] = None, **kw) -> Tensor:
-        """Variable-length clips (float32 or int16 PCM) in HOST memory, pad()ded to ``max_len`` on the device, HOST
-        features out (see ``FrontEndEngine.features_host_ragged``)."""
-        return self.engine.features_host_ragged(flat_host, offsets, lengths, int(max_len), out_host, **kw)
+                            out_host: Optional[Tensor] = None, *, pad: str = "repeat", **kw) -> Tensor:
+        """Variable-length clips (float32 or int16 PCM) in HOST memory, repeat- or zero-padded (``pad``) to ``max_len``
+        on the device, HOST features out (see ``FrontEndEngine.features_host_ragged``)."""
+        return self.engine.features_host_ragged(flat_host, offsets, lengths, int(max_len), out_host, pad=pad, **kw)
 
 
 class Spectrogram(nn.Module):

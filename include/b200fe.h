@@ -56,6 +56,15 @@ typedef enum b200fe_variant {
   B200FE_VARIANT_DFT_GEMM = 2    /* folded DFT as a split-fp16 GEMM on tcgen05 tensor cores / TMEM   */
 } b200fe_variant;
 
+/* How a ragged clip shorter than T becomes a T-sample row (the pad_mode argument of the *_pad entry points).
+ * A clip of at least T samples keeps its first T samples in both modes.  Pre-emphasis, when set, runs over the
+ * T-sample row, then torch.stft's reflect padding. */
+typedef enum b200fe_pad_mode {
+  B200FE_PAD_REPEAT = 0,         /* sample i = clip[i mod len]: the training loader's pad() (maze5.py:280-285)       */
+  B200FE_PAD_ZERO = 1            /* sample i = clip[i] for i < len, then 0.0f: the evaluation script's dataset
+                                    (Maze5_eval.py:203-221); with pre-emphasis y[len] = -a*clip[len-1], later 0     */
+} b200fe_pad_mode;
+
 /* Everything that fixes the transform.  Mirrors the constructor arguments of torchaudio's
  * Spectrogram / LFCC / MelSpectrogram / ComputeDeltas (transforms/_transforms.py:25,721,515,992). */
 typedef struct b200fe_params {
@@ -126,6 +135,8 @@ int64_t b200fe_workspace_bytes(const b200fe_params* p, int64_t R, int64_t T);
  * (ragged clips of at least T samples whose first sample is 16-byte aligned are read in place instead; the
  * workspace size does not depend on how many there are). */
 int64_t b200fe_workspace_bytes_ex(const b200fe_params* p, int64_t R, int64_t T, int32_t ragged);
+/* The sizers of ragged calls (b200fe_workspace_bytes_ex with ragged != 0, b200fe_workspace_bytes_ragged_i16,
+ * b200fe_host_staging_bytes_ragged) serve both pad modes: zero-padding stages exactly the rows repeat-padding stages. */
 
 /* The ragged call of b200fe_features_forward with 16-bit PCM clips, what the reference's loader decodes before it turns
  * them into float32 and pad()s them (maze5.py:297-351, :280-285): every row is staged as a dense float32 row in the
@@ -156,6 +167,20 @@ int32_t b200fe_spectrogram_forward(const float* wave, int64_t R, int64_t T, cons
 int32_t b200fe_features_forward(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
                                 const int32_t* lengths, const b200fe_params* p, const void* tables,
                                 float* out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* The ragged calls with a choice of padding: b200fe_features_forward (offsets and lengths required here) and
+ * b200fe_features_forward_ragged_i16 with pad_mode (b200fe_pad_mode) after the clip table.  B200FE_PAD_REPEAT is the
+ * call without the suffix; B200FE_PAD_ZERO zero-pads clips shorter than T.  The same kernels are launched and the same
+ * rows staged in both modes, so the workspace sizes are those of the calls without the suffix.  A pad_mode outside
+ * {0, 1} returns B200FE_ERR_BAD_ARG before any CUDA call. */
+int32_t b200fe_features_forward_ragged_pad(const float* wave, int64_t R, int64_t T, const int64_t* offsets,
+                                           const int32_t* lengths, int32_t pad_mode, const b200fe_params* p,
+                                           const void* tables, float* out, void* workspace, size_t workspace_bytes,
+                                           void* stream);
+int32_t b200fe_features_forward_ragged_i16_pad(const int16_t* pcm, int64_t R, int64_t T, const int64_t* offsets,
+                                               const int32_t* lengths, int32_t pad_mode, const b200fe_params* p,
+                                               const void* tables, float* out, void* workspace, size_t workspace_bytes,
+                                               void* stream);
 
 /* Stage output of the same path: the filterbank energies (spec^T @ fb)^T of
  * transforms/_transforms.py:818, before log / DCT / deltas:  out float32 device [R][n_filter][n_frames].
@@ -222,6 +247,14 @@ int32_t b200fe_features_forward_host_ragged(const void* clips_host, int32_t samp
                                             int64_t T, const b200fe_params* p, const void* tables, float* out_host,
                                             void* staging, size_t staging_bytes, int64_t chunk_rows,
                                             void* const* streams, int32_t n_streams);
+/* The same with pad_mode (b200fe_pad_mode) after the clip table; B200FE_PAD_REPEAT is the call above.  The chunks,
+ * copies, launches and staging size are the same in both modes. */
+int32_t b200fe_features_forward_host_ragged_pad(const void* clips_host, int32_t sample_bytes, int64_t n_samples,
+                                                const int64_t* offsets_host, const int32_t* lengths_host,
+                                                int32_t pad_mode, int64_t R, int64_t T, const b200fe_params* p,
+                                                const void* tables, float* out_host, void* staging,
+                                                size_t staging_bytes, int64_t chunk_rows, void* const* streams,
+                                                int32_t n_streams);
 
 /* ---- scoring tail on the device (SURVEY 8f-2) ---------------------------------------------------
  * Replaces the host-side  fpr, tpr, thr = sklearn.metrics.roc_curve(y, s); fnr = 1 - tpr;
